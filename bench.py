@@ -11,6 +11,9 @@ poses inside the timed region).  At N = 1 the same line also carries BASELINE co
 B = 1 latency of the DragPoserDLL C ABI (`latency`).  `--impl reference` times the CPU
 oracle port of the reference loop (the reference is Python and cannot travel to the GPU
 box) on all host cores.  One JSON line on stdout (rank 0).
+`--dump-outputs DIR` also writes the results of the last timed step (DIR/pose.npy,
+DIR/global_pos.npy; DIR/3trk_var_*.npy for config 3): the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -205,7 +208,9 @@ def dll_latency(calls=1000):
     class F2(C.Structure):
         _fields_ = [("x", C.c_float), ("y", C.c_float)]
 
-    lib = C.CDLL(build.build_all()[1])
+    if not os.path.exists(build.DLL_SO):  # built by build(); the benchmark compiles nothing (its tree may be read-only)
+        raise SystemExit(f"bench.py: {build.DLL_SO} is missing: build it first (python -m dragposer_b200.build)")
+    lib = C.CDLL(build.DLL_SO)
     V = C.c_void_p
     lib.init_drag_poser.restype = V
     lib.set_reference_skeleton.argtypes = [V, C.c_char_p]
@@ -307,7 +312,7 @@ def run_reference(args):
     if rank != 0:
         return
     cfg = get_config(args.trackers)
-    n_warm, n_timed = max(1, min(args.warmup, 1)), max(1, min(args.steps, 8))
+    n_warm, n_timed = max(1, min(args.warmup, 1)), max(1, args.steps)
     value, cores, sample = cpu_reference(n_warm, n_timed, args.trackers)
     config = workload_config(args, cfg, args.clips * args.gpus)
     # what this arm actually ran: per-clip CPU cost does not depend on how many clips exist, so the bounded sample stands for the
@@ -425,6 +430,12 @@ def measure(args, trackers, K, W, rank, world, dev, local, clocks=None):
     ms_pred, ms_frame, nprof = eng.profile()
     eng.set_profiling(False)
     clk = clocks.stop() if clocks is not None else None
+    # rows [pose 88 | global_pos 3] of the last timed step as its consumer receives them (rank 0 holds every rank's rows); copied
+    # here because the e2e pass below reuses the gather buffers
+    last_rows = None
+    if args.dump_outputs and rank == 0:
+        rows = dpdist.GatheredFrames(recv[-1], n_total).frame(0) if world > 1 else d_rows[W + K - 1]
+        last_rows = rows[:, :91].cpu().numpy()
     ms_by_rank, parts_by_rank = [ms / K], None
     if world > 1:
         dist.barrier()
@@ -527,7 +538,7 @@ def measure(args, trackers, K, W, rank, world, dev, local, clocks=None):
     torch.cuda.set_stream(torch.cuda.default_stream(dev))
     return dict(cfg=cfg, value=value, ms=ms, K=K, launches=launches, frame_ms=ms_frame / max(nprof, 1), pred_ms=ms_pred / max(nprof, 1), clk=clk,
                 ms_by_rank=ms_by_rank, parts_by_rank=parts_by_rank, e2e_value=n_total * K / e2e_s, h2d=h2d, d2h=d2h, path=path, n_total=n_total,
-                e2e_gathered=(n_total * K / e2e_gathered_s) if world > 1 else None,
+                e2e_gathered=(n_total * K / e2e_gathered_s) if world > 1 else None, last_rows=last_rows,
                 gather={"chunks": n_chunks, "to": "rank 0", "bytes_received_by_rank_0": int(max(world - 1, 0) * K * B * dpdist.ROW * 4)})
 
 
@@ -545,6 +556,22 @@ def roofline(m, B, trackers, peaks):
             "tensor_pipe_pct_of_peak_ncu": {"dp_frame_tc16_kernel": 12.12, "tp_ff_tc_kernel": 53.9, "tp_attn_tc_kernel": 7.26,
                                             "source": "profiles/r2_frame_kernel.md, r2_predictor.md: sm__ops_path_tensor_op_utchmma_src_fp16_dst_fp32 (issued ops, % of peak sustained elapsed)"},
             "note": "dependency-latency bound path (SURVEY 8d): both fractions are small by construction"}
+
+
+DUMP_BYTES = 63 << 20  # all arrays of one dump together, below 64 MB with room for the .npy headers
+
+
+def dump_outputs(out_dir, rows_by_prefix):
+    """Writes <prefix>pose.npy (n,88) and <prefix>global_pos.npy (n,3), float32, per workload: the last timed step's results, so
+    that two builds run with the same arguments can be compared output for output.  Above the byte budget a fixed, seeded sample
+    of clips (the same one on every run) is written, in clip order."""
+    os.makedirs(out_dir, exist_ok=True)
+    keep = DUMP_BYTES // len(rows_by_prefix) // (91 * 4)
+    for prefix, rows in rows_by_prefix.items():
+        if rows.shape[0] > keep:
+            rows = rows[np.sort(np.random.default_rng(0).choice(rows.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{prefix}pose.npy"), np.ascontiguousarray(rows[:, :88], np.float32))
+        np.save(os.path.join(out_dir, f"{prefix}global_pos.npy"), np.ascontiguousarray(rows[:, 88:91], np.float32))
 
 
 def run_ours(args):
@@ -585,17 +612,23 @@ def run_ours(args):
             line["gather"] = m["gather"]
             line["e2e"]["delivery"] = "every rank reads its own result rows into its own pinned host memory (the caller keeps shards)"
             line["e2e"]["gathered_to_rank0_value"] = m["e2e_gathered"]  # the same K steps with all rows gathered into rank 0's host memory
+    outputs = {"": m["last_rows"]}
     if world == 1 and not args.no_config3 and args.trackers == "6":
         # BASELINE config 3 in the same record: head + hands with the hands dropping out, window 16 (the predictor runs on every 16th
-        # frame with five decoder passes), 4096 clips; at least 32 frames so that two predictor frames fall into the timed region
-        k3 = max(K, 32)
-        m3 = measure(args, "3", k3, W, rank, world, dev, local)
+        # frame with five decoder passes), 4096 clips.  The per-step cost depends on how many predictor frames (t % 16 == 0) fall
+        # into the K timed frames W..W+K-1: a multiple of 16 for --steps weighs them as a long run does, and the record says how many
+        m3 = measure(args, "3", K, W, rank, world, dev, local)
+        outputs["3trk_var_"] = m3["last_rows"]
+        window = m3["cfg"].temporal_future_window
         line["configs"] = {("3trk_var_4096" if args.clips == 4096 else f"3trk_var_{args.clips}"): {
-            "value": m3["value"], "unit": "clip-frames/s", "steps": k3, "ms_per_step": m3["ms"] / k3,
+            "value": m3["value"], "unit": "clip-frames/s", "steps": K, "ms_per_step": m3["ms"] / K,
+            "predictor_steps": sum(1 for t in range(W, W + K) if t % window == 0),
             "config": workload_config(args, m3["cfg"], m3["n_total"], "3"), "roofline": roofline(m3, args.clips, "3", peaks),
             "e2e": {"value": m3["e2e_value"], "unit": "clip-frames/s", "h2d_bytes_per_step": m3["h2d"], "d2h_bytes_per_step": m3["d2h"]},
             "gpu_launches": m3["launches"]}}
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         if world == 1 and not args.no_latency:
             line["latency"] = dll_latency()
         if world == 1 and not args.no_cpu_baseline:
@@ -619,7 +652,10 @@ def main():
     ap.add_argument("--no-latency", action="store_true", help="skip the B = 1 C-ABI latency measurement")
     ap.add_argument("--no-config3", action="store_true", help="skip the second workload (BASELINE config 3) at N = 1")
     ap.add_argument("--decoder-path", type=int, default=0, choices=[0, 1, 3], help="0 auto, 1 fp32 CUDA-core decoder, 3 tcgen05 fp16x2")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the poses and root positions of the last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

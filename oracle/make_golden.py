@@ -216,6 +216,19 @@ def golden_temporal(ref):
     np.savez_compressed(os.path.join(OUT, "ref_temporal.npz"), **out)
 
 
+def golden_temporal_pt_layout(ref):
+    """What train_temporal.load_model (train_temporal.py:474-482) reads from temporal.pt: the checkpoint's keys (train.py:311-319),
+    the shapes of the latent statistics and the names and shapes of the reference Temporal module's state dict, which
+    load_state_dict requires exactly."""
+    import json
+
+    layout = {"checkpoint_keys": ["model_state_dict", "means_latent", "stds_latent"], "means_latent": [24], "stds_latent": [24],
+              "model_state_dict": {k: list(v.shape) for k, v in ref.temporal.state_dict().items()}}
+    with open(os.path.join(OUT, "temporal_pt_layout.json"), "w") as fh:
+        json.dump(layout, fh, indent=1)
+        fh.write("\n")
+
+
 def golden_rundrag(ref):
     """The C-ABI session of DragPoserDLL/main.cpp:17-38 driven through the reference's
     RunDrag (run_drag.py) with the example skeleton: 6 frames, MaxIter 10, lr 0.01, window 60."""
@@ -498,7 +511,7 @@ def golden_eval_full(ref):
     eval_metrics.eval_pos_error, the per-frame iteration counts and root positions, and ships the clip itself gzip-compressed
     (motion data: CC BY-SA 4.0, LICENSE_data) so the GPU box can run the same evaluation."""
     import gzip
-    import shutil
+    import io
     import time
 
     n_frames = ref.rots.shape[0]
@@ -506,8 +519,13 @@ def golden_eval_full(ref):
     latent0, rp, rg, its, _ = _eval_loop(ref, n_frames, "example.bvh")
     secs = time.time() - t0
     mpjpe, mpeepe, _ = _reference_result_and_metrics(ref, rp, rg, os.path.dirname(rh.EXAMPLE_BVH), "example.bvh", n_frames)
-    with open(rh.EXAMPLE_BVH, "rb") as src, gzip.GzipFile(os.path.join(OUT, "example_full.bvh.gz"), "wb", compresslevel=9, mtime=0) as dst:
-        shutil.copyfileobj(src, dst)
+    packed = io.BytesIO()
+    with open(rh.EXAMPLE_BVH, "rb") as src, gzip.GzipFile("example_full.bvh.gz", "wb", 9, packed, mtime=0) as dst:
+        dst.write(src.read())
+    cut = 960000  # the gzip file in two pieces, each below 1 MB; `cat example_full.bvh.gz.1 example_full.bvh.gz.2` rejoins them
+    for i, part in enumerate((packed.getvalue()[:cut], packed.getvalue()[cut:]), 1):
+        with open(os.path.join(OUT, f"example_full.bvh.gz.{i}"), "wb") as fh:
+            fh.write(part)
     np.savez_compressed(os.path.join(OUT, "ref_eval_full.npz"), latent0=latent0, mpjpe=np.float64(mpjpe), mpeepe=np.float64(mpeepe),
                         iters=its.astype(np.int16), gpos=rg[0].numpy().T.copy(), pose_every_100=rp[0].numpy().T[::100].copy(),
                         seconds_one_core=np.float64(secs))
@@ -519,13 +537,15 @@ if __name__ == "__main__":
     torch.set_num_threads(1)
     ref = build()
     pm = save_model_fixture(ref)
-    which = sys.argv[1:] or ["trace", "frames3", "temporal", "rundrag", "evalbvh", "encoder", "resultpath", "extlosses"]
+    which = sys.argv[1:] or ["trace", "frames3", "temporal", "tplayout", "rundrag", "evalbvh", "encoder", "resultpath", "extlosses"]
     if "trace" in which:
         golden_iter_traces(ref, pm)
     if "frames3" in which:
         golden_frames_3trk(ref, pm)
     if "temporal" in which:
         golden_temporal(ref)
+    if "tplayout" in which:
+        golden_temporal_pt_layout(ref)
     if "rundrag" in which:
         golden_rundrag(ref)
     if "evalbvh" in which:

@@ -101,6 +101,29 @@ def test_temporal_pt_round_trip_in_reference_format(tmp_path, temporal_model):
     assert np.array_equal(flat[-48:-24], tm.means_latent) and np.array_equal(flat[-24:], tm.stds_latent)
 
 
+def test_temporal_pt_has_the_layout_the_reference_loader_reads(tmp_path, temporal_model):
+    """A file written by save_temporal_model holds what the reference's train_temporal.load_model (train_temporal.py:474-482) reads:
+    the checkpoint keys, the latent statistics, and a state dict with the names and shapes of the reference Temporal module
+    (golden/temporal_pt_layout.json, recorded by `python -B oracle/make_golden.py tplayout`), which its strict load_state_dict
+    requires."""
+    import json
+
+    from dragposer_b200 import model
+
+    with open(os.path.join(G, "temporal_pt_layout.json")) as fh:
+        layout = json.load(fh)
+    tm = model.TemporalModel(temporal_model.sd, np.full(24, 0.25, np.float32), np.full(24, 2.0, np.float32))
+    path = str(tmp_path / "temporal.pt")
+    model.save_temporal_model(tm, path)
+    ck = torch.load(path, map_location="cpu")
+    assert sorted(ck) == sorted(layout["checkpoint_keys"])
+    assert {k: list(v.shape) for k, v in ck["model_state_dict"].items()} == layout["model_state_dict"]
+    for k, v in ck["model_state_dict"].items():
+        assert v.dtype == torch.float32 and np.array_equal(v.numpy(), tm.sd[k]), k
+    for name, value in (("means_latent", 0.25), ("stds_latent", 2.0)):
+        assert list(ck[name].shape) == layout[name] and ck[name].dtype == torch.float32 and torch.all(ck[name] == value), name
+
+
 def test_temporal_pt_loads_into_the_reference_module(tmp_path, temporal_model):
     """When the reference tree is present: the file written by save_temporal_model is accepted by the reference's own
     train_temporal.load_model (train_temporal.py:474-482)."""

@@ -253,3 +253,30 @@ def test_headline_3_trackers_early_stop_iteration_counts_vs_oracle(engine_factor
     print(f"3 trackers, early stop, {T} frames x {len(idx)} sampled clips: {checked} clip-frames compared (iterations +-1, positions <= 1 mm), "
           f"{slipped} clips left after a +-1 slip of the stop decision, {dropped_ill} left as ill-conditioned; mean {mean_it:.1f} iterations per frame")
     assert checked >= 0.5 * T * len(idx)
+
+
+@pytest.mark.parametrize("trackers", ["6", "3"])
+def test_bench_keeps_the_last_timed_step_in_clip_order(pose_model, model_npz, temporal_model, trackers):
+    """What bench.py --dump-outputs writes (measure()'s `last_rows`) is the last timed step, clip by clip: bitwise the rows
+    BatchedDragPose.run_frames gives for that frame of the same seeded workload from the same start."""
+    import argparse
+
+    import bench
+    from dragposer_b200.engine import BatchedDragPose, RunOptions
+
+    n, W, K = 600, 3, 3  # >= 512 clips: the tcgen05 frame kernel, as at the headline size
+    m = bench.measure(argparse.Namespace(clips=n, decoder_path=0, dump_outputs="-"), trackers, K, W, 0, 1, torch.device("cuda", 0), 0)
+    cfg = bench.get_config(trackers)
+    wl = synthetic.make_workload(pose_model, model_npz["offsets"], cfg, n, W + K, variable_mask=trackers == "3")
+    eng = BatchedDragPose(pose_model, model_npz["offsets"], temporal_model, n)
+    eng.set_initial_state(wl["latent0"], np.zeros((n, 3)), np.tile([[1.0, 0, 0, 0]], (n, 1)), np.zeros((n, 6)))
+    opts = RunOptions(decoder_path=0, **bench.fixed_opts(cfg))
+    if trackers == "3":
+        pose, gpos = eng.run_frames(wl["tgt_pos"], wl["tgt_rot"], wl["joints_tb"], wl["weights_tb"], n_ee=wl["n_ee"], options=opts)
+    else:
+        pose, gpos = eng.run_frames(wl["tgt_pos"], wl["tgt_rot"], wl["joints"], wl["weights"], options=opts)
+    eng.close()
+    want = np.concatenate([pose[-1], gpos[-1]], 1)
+    err, step_apart = np.abs(m["last_rows"] - want).max(), np.abs(np.concatenate([pose[-2], gpos[-2]], 1) - want).max()
+    print(f"{trackers} trackers: last timed step vs run_frames max diff {err:.2e} (neighbouring steps differ by {step_apart:.2e})")
+    assert m["last_rows"].shape == (n, 91) and err == 0 < step_apart

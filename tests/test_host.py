@@ -182,3 +182,22 @@ def test_engine_fails_loudly_without_library(monkeypatch, tmp_path):
     monkeypatch.setattr(_lib, "ENGINE_SO", str(tmp_path / "nope.so"))
     with pytest.raises(_lib.EngineError, match="no CPU fallback"):
         _lib.load()
+
+
+def test_bench_output_dump_is_a_fixed_sample_below_64_mb(tmp_path):
+    """bench.py --dump-outputs: every clip while they fit; above that the same seeded sample of clips on every run, in clip order,
+    with all arrays of one dump together below 64 MB."""
+    import bench
+
+    small = np.arange(5 * 91, dtype=np.float32).reshape(5, 91)
+    bench.dump_outputs(str(tmp_path / "a"), {"": small})
+    assert np.array_equal(np.load(tmp_path / "a" / "pose.npy"), small[:, :88])
+    assert np.array_equal(np.load(tmp_path / "a" / "global_pos.npy"), small[:, 88:91])
+    big = np.repeat(np.arange(200_000, dtype=np.float32)[:, None], 91, 1)  # row c holds c; 73 MB per workload
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"": big, "3trk_var_": big})
+    assert sum(f.stat().st_size for f in (tmp_path / "b").iterdir()) <= 64 << 20
+    for name in ("pose", "global_pos", "3trk_var_pose", "3trk_var_global_pos"):
+        x, y = np.load(tmp_path / "b" / f"{name}.npy"), np.load(tmp_path / "c" / f"{name}.npy")
+        assert x.dtype == np.float32 and np.array_equal(x, y)
+    assert (np.diff(np.load(tmp_path / "b" / "pose.npy")[:, 0]) > 0).all()

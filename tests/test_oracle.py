@@ -84,6 +84,27 @@ def test_rundrag_local_quaternion_conversion(golden_dir, port_weights):
     assert np.allclose(np.linalg.norm(q, axis=-1), 1.0, atol=1e-4)
 
 
+def test_port_matches_recorded_reference_one_frame(golden_dir, port_weights, temporal_model):
+    """The one-frame comparison below (fresh start, early-stop thresholds capped at 25 iterations, seed-2222 predictor) against the
+    reference's recorded run of frame 0 (ref_trace_6trk.npz): each clip ran past 25 iterations there, so a capped reference run is
+    exactly those first 25 iterations, and the port must follow that latent path and its losses."""
+    g = np.load(os.path.join(golden_dir, "ref_trace_6trk.npz"))
+    cfg = synthetic.config_6_trackers()
+    B, n = g["latent0"].shape[0], 25
+    assert (g["early_iters"][0] > n).all()
+    d = port.PortDragPose(port_weights, temporal_model.sd)
+    d.set_initial_state(g["latent0"], np.zeros((B, 3)), np.tile([[1.0, 0, 0, 0]], (B, 1)), np.zeros((B, 6)))
+    d.trace = []
+    d.run(g["tgt_pos"][0], g["tgt_rot"][0], g["joints"], g["weights"], lambda_rot=1.0, lambda_temporal=cfg.lambda_temporal,
+          temporal_future_window=0, joint_adjustment=cfg.joint_adjustment, joint_adjustment_weight=cfg.joint_adjustment_weight,
+          **dict(EARLY, max_iter=n))
+    assert (d.iters.numpy() == n).all() and len(d.trace) == n
+    latents = np.stack([r["latent"] for r in d.trace], 1)
+    assert np.abs(latents - g["early_latent"][0, :, :n]).max() < 2e-5
+    np.testing.assert_allclose(np.stack([r["lp"] for r in d.trace], 1), g["early_loss"][0, :, :n, 0], rtol=1e-4, atol=1e-9)
+    np.testing.assert_allclose(np.stack([r["lr"] for r in d.trace], 1), g["early_loss"][0, :, :n, 1], rtol=1e-4, atol=1e-9)
+
+
 @pytest.mark.skipif(not rh.available(), reason="live reference only exists in the build container")
 def test_port_matches_live_reference_one_frame(port_weights, pose_model, model_npz):
     from dragposer_b200 import model as dpm
