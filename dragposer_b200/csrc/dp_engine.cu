@@ -40,7 +40,7 @@ struct dp_engine {
   float* d_tblob = nullptr;
   unsigned char* d_fftiles = nullptr;  // pre-tiled fp16x2 tensor-core weight images of the predictor (DP_TC_TILES_BYTES)
   int predictor_path = 0;              // 0 = tcgen05 FF (default), 1 = fp32 CUDA-core FF
-  int last_path = 0;                   // decoder path of the last frame: 1 = fp32, 2 = tcgen05
+  int last_path = 0;                   // decoder path of the last frame: 1 = fp32, 3 = tcgen05 fp16x2
   float *d_mu = nullptr, *d_sigma = nullptr;
   TpLayout tl;
   // state
@@ -54,7 +54,6 @@ struct dp_engine {
   // (train_temporal.param["past_frames"] stops at ring row 56 of 60), so the targets of this frame AND the next three are computed
   // in ONE batched predictor call (4 x n_clips virtual clips: fuller tiles, a quarter of the launches) -- the same numbers the
   // reference computes frame by frame.
-  int lookahead = DP_LOOKAHEAD;   // 1 disables (environment DP_LOOKAHEAD=1)
   float* d_target_pre = nullptr;  // (B, DP_LOOKAHEAD, 24)
   int look_left = 0, look_next = 0, look_last_row = -1;
   // Predictor ahead of time in the small-batch streaming mode (window >= 4, <= DP_PREFETCH_MAX_CLIPS clips; DP_PRED_PREFETCH=0 turns it
@@ -139,7 +138,6 @@ extern "C" int dp_engine_create(dp_engine** out, int device, int max_clips) {
   CK(cudaMalloc(&e->d_losses, B * 3 * 4));
   CK(cudaMalloc(&e->d_mu, DP_L * 4));
   CK(cudaMalloc(&e->d_sigma, DP_L * 4));
-  if (const char* s = getenv("DP_LOOKAHEAD")) e->lookahead = atoi(s) <= 1 ? 1 : DP_LOOKAHEAD;
   const size_t V = B * DP_LOOKAHEAD;  // virtual clips of a look-ahead predictor call
   CK(cudaMalloc(&e->d_target_pre, V * DP_L * 4));
   CK(cudaMemset(e->d_target_pre, 0, V * DP_L * 4));
@@ -157,10 +155,8 @@ extern "C" int dp_engine_create(dp_engine** out, int device, int max_clips) {
   CK(cudaEventCreateWithFlags(&e->ev_pre_fork, cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&e->ev_pre_done, cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&e->tw.ev_fork, cudaEventDisableTiming));
-  for (int i = 0; i < DP_PRED_MAX_PARTS - 1; ++i) {
-    CK(cudaStreamCreateWithFlags(&e->tw.st_extra[i], cudaStreamNonBlocking));
-    CK(cudaEventCreateWithFlags(&e->tw.ev_join[i], cudaEventDisableTiming));
-  }
+  CK(cudaStreamCreateWithFlags(&e->tw.st_extra, cudaStreamNonBlocking));
+  CK(cudaEventCreateWithFlags(&e->tw.ev_join, cudaEventDisableTiming));
   *out = e;
   return DP_OK;
 }
@@ -187,8 +183,8 @@ extern "C" int dp_engine_destroy(dp_engine* e) {
   cudaFree(e->d_disp_buf); cudaFree(e->d_height_buf); cudaFree(e->d_target_buf); cudaFree(e->d_target_pre); cudaFree(e->d_iters);
   cudaFree(e->d_losses); cudaFree(e->d_trace); cudaFree(e->d_adam); cudaFree(e->d_phase);
   cudaFree(e->tw.enc); cudaFree(e->tw.enc2); cudaFree(e->tw.dec); cudaFree(e->tw.dec2); cudaFree(e->tw.dec_lat); cudaFree(e->tw.ffpart);
-  for (int i = 0; i < DP_PRED_MAX_PARTS - 1; ++i)
-    if (e->tw.st_extra[i]) { cudaStreamSynchronize(e->tw.st_extra[i]); cudaStreamDestroy(e->tw.st_extra[i]); cudaEventDestroy(e->tw.ev_join[i]); }
+  if (e->tw.st_extra) { cudaStreamSynchronize(e->tw.st_extra); cudaStreamDestroy(e->tw.st_extra); }
+  if (e->tw.ev_join) cudaEventDestroy(e->tw.ev_join);
   if (e->tw.ev_fork) cudaEventDestroy(e->tw.ev_fork);
   if (e->pre_stream) { cudaStreamSynchronize(e->pre_stream); cudaStreamDestroy(e->pre_stream); }
   if (e->ev_pre_fork) cudaEventDestroy(e->ev_pre_fork);
@@ -467,7 +463,7 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
     for (int i = 0; i < 3; ++i) CK(cudaEventCreate(&ev[i]));
     CK(cudaEventRecord(ev[0], st));
   }
-  const bool look = W == 0 && e->lookahead > 1;
+  const bool look = W == 0;
   if (!look) {
     e->look_left = 0;
     e->look_last_row = -1;
@@ -497,12 +493,12 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
     }
   } else {
     drop_prefetch(e);
-    if (e->look_left == 0) {  // targets of this frame and of the next lookahead - 1 frames in one call
+    if (e->look_left == 0) {  // targets of this frame and of the next DP_LOOKAHEAD - 1 frames in one call
       if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
       CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_latent_buf, e->d_disp_buf, e->d_height_buf,
                          e->ring_head, e->n_clips, 0, e->d_target_pre, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles, st,
-                         &e->launches, e->lookahead));
-      e->look_left = e->lookahead;
+                         &e->launches, DP_LOOKAHEAD));
+      e->look_left = DP_LOOKAHEAD;
       e->look_next = 0;
     }
     e->look_last_row = e->look_next++;
@@ -524,7 +520,7 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
   a.latent_buf = e->d_latent_buf; a.disp_buf = e->d_disp_buf; a.height_buf = e->d_height_buf;
   a.ring_head = e->ring_head;
   a.target_buf = e->d_target_buf; a.target_rows = W + 1; a.target_index = e->current_index;
-  if (look) { a.target_buf = e->d_target_pre; a.target_rows = e->lookahead; a.target_index = e->look_last_row; }
+  if (look) { a.target_buf = e->d_target_pre; a.target_rows = DP_LOOKAHEAD; a.target_index = e->look_last_row; }
   a.n_ee = n_ee; a.joints = joints; a.weights = weights; a.shared_trackers = shared;
   a.tgt_pos = tgt_pos; a.tgt_rot = tgt_rot; a.ee_stride = ee_stride;
   a.targets_world = p->targets_world ? 1 : 0;
@@ -908,7 +904,7 @@ extern "C" int dp_engine_get_state(dp_engine* e, float* latent, float* gpos, flo
   if (target_buf) {
     if (e->target_rows <= 0) return fail(DP_ERR_STATE, "no target buffer yet");
     if (e->look_last_row >= 0)  // window 0 with look-ahead: the row the last frame used, as (B,1,24)
-      CK(cudaMemcpy2D(target_buf, DP_L * 4, e->d_target_pre + (size_t)e->look_last_row * DP_L, (size_t)e->lookahead * DP_L * 4, DP_L * 4, B,
+      CK(cudaMemcpy2D(target_buf, DP_L * 4, e->d_target_pre + (size_t)e->look_last_row * DP_L, (size_t)DP_LOOKAHEAD * DP_L * 4, DP_L * 4, B,
                       cudaMemcpyDeviceToHost));
     else
       CK(cudaMemcpy(target_buf, e->d_target_buf, B * e->target_rows * DP_L * 4, cudaMemcpyDeviceToHost));

@@ -1,16 +1,16 @@
 // dp_frame_tc16.cu -- persistent per-frame optimisation kernel, fp16x2 split products on tcgen05 with the WEIGHTS
 // resident in tensor memory (default path for batches).
 //
-// Same contract and arithmetic as dp_frame_tc.cu (one launch == one frame of DragPose.run, python/src/drag_pose.py:196-414,
-// for every clip; decoder forward 24->40->60->92 and its data-gradient as D[features x clips] = W . X tiles), restructured
+// One launch == one frame of DragPose.run (python/src/drag_pose.py:196-414) for every clip, the same contract as the fp32 kernel
+// (dp_frame_simt.cu); the decoder forward 24->40->60->92 and its data-gradient run as D[features x clips] = W . X tiles, built
 // around what the phase clock and the MMA-rate probes measured on B200:
 //   * an MMA whose A operand comes from shared memory costs ~41 cycles at N = 16 whatever the math; with A in tensor memory
 //     (TS mode) it costs ~12.  The six weight matrices (forward W_l and backward W_l^T, two fp16 pieces each, 16 W) fit in
 //     352 of the 512 tensor-memory columns, so they are loaded there once per launch and shared memory only carries the
 //     activations (B operand, MN-major).
-//   * the CUDA cores idle during the tensor phases and vice versa, so ONE CTA per SM runs TWO independent groups of
-//     8 warps x 16 clips.  Each group has its own accumulator columns, mbarrier, named block barrier and loop exit; they
-//     share the tensor-memory weights and drift apart naturally, one group's kinematics overlapping the other's layers.
+//   * the CUDA cores idle during the tensor phases and vice versa, so ONE CTA per SM runs FOUR independent groups of
+//     4 warps x 8 clips.  Each group has its own accumulator columns, mbarrier, named block barrier and loop exit; they
+//     share the tensor-memory weights and drift apart naturally, one group's kinematics overlapping the others' layers.
 //   * kinematics / loss / adjoint: two clips per warp in packed fp32x2 registers (dp_fk2.cuh); optimiser state in shared
 //     memory.
 #include "dp_fk2.cuh"
@@ -19,52 +19,38 @@
 
 namespace {
 
-#ifndef DP_TC16_GROUPS
-#define DP_TC16_GROUPS 4
-#endif
 constexpr int NC = 32;                     // clip columns per CTA
 constexpr int kWarps = 16;
-// DP_KIN_GATE=1: the groups form two teams (gid & 1) that take turns in the kinematics pass -- team 0 starts pass n when team 1 has
-// finished pass n - 1, team 1 starts pass n when team 0 has finished pass n -- so that a sub-partition never runs more than two of
-// the 971-instruction passes at once and one team's tensor phases lie under the other team's kinematics.
-#ifndef DP_KIN_GATE
-#define DP_KIN_GATE 0
-#endif
-constexpr bool kKinGate = DP_KIN_GATE && DP_TC16_GROUPS == 4;
-constexpr int kGroups = DP_TC16_GROUPS;    // independent clip groups of a CTA (2 or 4)
-constexpr int kGW = kWarps / kGroups;      // warps per group: 8 (16 clips) or 4 (8 clips)
+constexpr int kGroups = 4;                 // independent clip groups of a CTA
+constexpr int kGW = kWarps / kGroups;      // warps per group: 4 (8 clips)
 constexpr int kGC = NC / kGroups;          // clip columns per group
 constexpr int kG8 = kGC / 8;               // 8-clip groups per fp16 piece of a group
-static_assert(kGroups == 2 || kGroups == 4, "two groups of 8 warps or four groups of 4 warps");
-constexpr int EC = 8;             // clips per epilogue thread: a group's 8 warps = 4 TMEM lane quarters x 2 clip halves
-// activation image (B operand, MN-major, no swizzle).  The two fp16 pieces of a group's 16 clips lie SIDE BY SIDE along N, so that
-// one N = 32 instruction multiplies a weight piece with both of them: element (feature k, group g, piece p, clip n < 16) at
-//   (k / 8) * kB_LBO + (k % 8) * 16 + ((2 g + p) kG8 + n / 8) * kB_SBO + (n % 8) * 2 bytes   (kG8 = 8-clip groups per piece: 2 or 1).
+constexpr int EC = 8;             // clips per epilogue thread: a group's 4 warps are the 4 TMEM lane quarters, each thread takes all 8 clips
+// activation image (B operand, MN-major, no swizzle).  The two fp16 pieces of a group's 8 clips lie SIDE BY SIDE along N, so that
+// one N = 16 instruction multiplies a weight piece with both of them: element (feature k, group g, piece p, clip n < 8) at
+//   (k / 8) * kB_LBO + (k % 8) * 16 + ((2 g + p) kG8 + n / 8) * kB_SBO + (n % 8) * 2 bytes   (kG8 = 8-clip groups per piece: 1).
 // The K 8-groups are padded from 1024 to 1040 bytes: unpadded, every 8-group starts in the same bank and the 32 lanes of an
 // epilogue warp (consecutive features, one 16-byte store each) collide four ways; the pad moves each group on by four banks.
 constexpr uint32_t kB_SBO = 128, kB_PIECE = kG8 * kB_SBO;
 constexpr uint32_t kB_LBO = kB_SBO * 2 * (NC / 8) + 16;
 constexpr uint32_t kPingBytes = (64 / 8) * kB_LBO, kPongBytes = (96 / 8) * kB_LBO;  // both pieces
-// dL/dy image (B operand of the first backward layer only), K-MAJOR: element (group g, piece p, clip n < 16, feature k) at
+// dL/dy image (B operand of the first backward layer only), K-MAJOR: element (group g, piece p, clip n < 8, feature k) at
 //   ((2 g + p) kG8 + n / 8) * kD_SBO + (k / 8) * kD_LBO + (n % 8) * 16 + (k % 8) * 2 bytes,
 // so that the kinematics lane of joint j stores its four values dL/dy[4j .. 4j+3] of a clip as ONE 8-byte word per piece -- the
 // adjoint writes the tensor-core operand itself and the backward layers start after a single group barrier (round 1 wrote fp32
 // rows, and the epilogue warps re-read them transposed, split them and stored them behind a second barrier).  kD_LBO is padded
 // from 128 to 144 bytes for the same bank reason as kB_LBO.
 constexpr uint32_t kD_LBO = 144, kD_SBO = (96 / 8) * kD_LBO, kD_PIECE = kG8 * kD_SBO, kDyBytes = 2 * (NC / 8) * kD_SBO;
-constexpr float kWScale = 16.0f;  // the weight image holds 16 W; dL/dy is scaled per clip into [16, 32) (see dp_frame_tc.cu)
+// the weight image holds 16 W and dL/dy is scaled per clip into [16, 32) (dp_fk2.cuh, SCALE): exact powers of two for fp16's narrow
+// exponent range, undone in the epilogues and when dL/dz is read
+constexpr float kWScale = 16.0f;
 // Generic-proxy writes of an operand image (st.shared by the epilogue / kinematics / Adam threads) must be ordered before the
-// tensor core's async-proxy reads.  1 (default): the ONE issuing thread executes fence.proxy.async after the group barrier that made
-// the writes visible to it -- writer's st.shared -> (program order) barrier arrive -> (synchronizes with) issuer's barrier ->
-// (program order) fence.proxy.async -> tcgen05.mma: the proxy fence lies on the base-causality path from the write to the read, which
-// is what the PTX memory model asks for; the barrier has drained the stores, so the fence is cheap.  0: every writer fences before
-// the barrier (the pattern of CUTLASS's TMA-store epilogues; MEMBAR.ALL.CTA with the warp's stores still in flight, 50-110 cycles
-// in each of the 7 hand-offs of an iteration).  Measured (scripts/ab_frame.sh, ms per frame at 4 096 clips): four groups 0.629 vs
-// 0.641; two groups 0.664 vs 0.666.  The whole GPU suite (bitwise permutation test included) passes either way.
-#ifndef DP_ISSUER_FENCE
-#define DP_ISSUER_FENCE 1
-#endif
-constexpr bool kIssuerFence = DP_ISSUER_FENCE != 0;
+// tensor core's async-proxy reads: the ONE issuing thread executes fence.proxy.async after the group barrier that made the writes
+// visible to it -- writer's st.shared -> (program order) barrier arrive -> (synchronizes with) issuer's barrier -> (program order)
+// fence.proxy.async -> tcgen05.mma: the proxy fence lies on the base-causality path from the write to the read, which is what the
+// PTX memory model asks for; the barrier has drained the stores, so the fence is cheap.  Every writer fencing before the barrier
+// (the pattern of CUTLASS's TMA-store epilogues; MEMBAR.ALL.CTA with the warp's stores still in flight, 50-110 cycles in each of
+// the 7 hand-offs of an iteration) measured 0.641 against 0.629 ms per frame at 4 096 clips (DESIGN.md section 3.1).
 enum { ST_Z = 0, ST_TL = 1, ST_M = 2, ST_V = 3, ST_ZLAST = 4 };
 // tensor-memory columns: accumulators of group g at 2 kGC g (kGC columns per B piece); then the weight pieces (two K elements per word)
 constexpr uint32_t kT_D = 0, kT_W = 64, kT_COLS = 512;
@@ -88,7 +74,6 @@ struct SmemT {
   int iters[NC];
   uint64_t bar_w, bar_mma[kGroups];
   uint32_t tmem_base;
-  uint32_t kin_done[2];                             // kinematics passes finished by the groups of a team (DP_KIN_GATE)
   __device__ __forceinline__ const DpModelImageTC& M() const { return *reinterpret_cast<const DpModelImageTC*>(model); }
 };
 
@@ -179,30 +164,29 @@ struct Ctx {
 
 // MMAs of one dense layer of one group; every thread of the group calls this, one elected lane of the group's first warp issues.
 // A = weight pieces in tensor memory, B = the group's clip columns of the activation image: per K step of 16
-//   D[:, 0..31] (+)= A1 . [B1 | B2]   (N = 32: the (1,1) product lands in columns 0..15, the (1,2) product in columns 16..31)
-//   D[:, 0..15]  += A2 . B1           (N = 16: the (2,1) product)
+//   D[:, 0..15] (+)= A1 . [B1 | B2]   (N = 16: the (1,1) product lands in columns 0..7, the (1,2) product in columns 8..15)
+//   D[:, 0..15]  += A2 . [B1 | B2]    (N = 16: the (2,1) product)
 // and the epilogue adds the two column blocks -- two instructions per K step instead of three (an instruction costs ~20 issue
-// cycles whatever its N).  B_KMAJOR: the B operand is the K-major dL/dy image instead of an MN-major activation image.
+// cycles whatever its N).  The second instruction takes both pieces as well because an M = 128 instruction needs N >= 16: it adds
+// the (2,2) product, a term of relative size 2^-22, to the second column block.  B_KMAJOR: the B operand is the K-major dL/dy
+// image instead of an MN-major activation image.
 template <int L, bool FWD, bool B_KMAJOR = false>
 __device__ __forceinline__ void tc_issue(Ctx& c, const unsigned char* src) {
   if (c.wg == 0) {
     tc_fence_after();
     if (elect_one()) {
-      if (kIssuerFence) fence_proxy_async();  // see kIssuerFence
-      // fp16 x fp16 -> fp32, M 128; bit 16: B is MN-major
-      constexpr uint32_t idesc = (1u << 4) | (B_KMAJOR ? 0u : (1u << 16)) | (8u << 24);
-      // both pieces: N = 2 kGC; first piece only: N = kGC -- but an M = 128 instruction needs N >= 16, so four groups of 8 clips issue the
-      // second instruction on both pieces as well (it adds the (2,2) product, a term of relative size 2^-22, to the second column block)
-      constexpr uint32_t idesc32 = idesc | ((uint32_t)((2 * kGC) >> 3) << 17), idesc16 = idesc | ((uint32_t)((kGC >= 16 ? kGC : 2 * kGC) >> 3) << 17);
+      fence_proxy_async();  // orders the group's st.shared operand writes before the MMAs (see "Generic-proxy writes" above)
+      // fp16 x fp16 -> fp32, M 128, N = 2 kGC; bit 16: B is MN-major
+      constexpr uint32_t idesc = (1u << 4) | (B_KMAJOR ? 0u : (1u << 16)) | ((uint32_t)((2 * kGC) >> 3) << 17) | (8u << 24);
       constexpr uint32_t lbo = B_KMAJOR ? kD_LBO : kB_LBO, sbo = B_KMAJOR ? kD_SBO : kB_SBO;
       const UmmaDescBase b = umma_desc_base(smem_u32(src) + (uint32_t)c.gid * 2 * kG8 * sbo, lbo, sbo);  // the group's 8-groups (both pieces)
       const uint32_t d = c.tmem + kT_D + 2 * kGC * c.gid, a1 = c.tmem + kT_W + WT<L, FWD>::p1, a2 = c.tmem + kT_W + WT<L, FWD>::p2;
 #pragma unroll
       for (int k = 0; k < (int)WT<L, FWD>::ksteps; ++k) {
         const uint32_t bo = k * 2 * lbo;  // K = 16 per instruction: two 8-groups of K
-        if (k == 0) umma_f16_ts_c<false>(d, a1 + 8 * k, umma_desc_at(b, bo), idesc32);
-        else umma_f16_ts_c<true>(d, a1 + 8 * k, umma_desc_at(b, bo), idesc32);
-        umma_f16_ts_c<true>(d, a2 + 8 * k, umma_desc_at(b, bo), idesc16);
+        if (k == 0) umma_f16_ts_c<false>(d, a1 + 8 * k, umma_desc_at(b, bo), idesc);
+        else umma_f16_ts_c<true>(d, a1 + 8 * k, umma_desc_at(b, bo), idesc);
+        umma_f16_ts_c<true>(d, a2 + 8 * k, umma_desc_at(b, bo), idesc);
       }
       umma_commit(&c.S->bar_mma[c.gid]);
     }
@@ -214,49 +198,47 @@ template <int L, bool FWD, bool B_KMAJOR = false, class Epi>
 __device__ __forceinline__ void tc_layer(Ctx& c, const unsigned char* src, int out_rows, Epi epi) {
   SmemT& S = *c.S;
   tc_issue<L, FWD, B_KMAJOR>(c, src);
-  const int quarter = c.wg & 3, half = c.wg >> 2;
+  const int quarter = c.wg & 3;
   if (quarter * 32 < out_rows) {
     mbar_wait(&S.bar_mma[c.gid], c.phase);
       tc_fence_after();
     float v[EC], w[EC];
-    const uint32_t t = c.tmem + ((uint32_t)(quarter * 32) << 16) + kT_D + (uint32_t)(2 * kGC * c.gid + EC * half);
+    const uint32_t t = c.tmem + ((uint32_t)(quarter * 32) << 16) + kT_D + (uint32_t)(2 * kGC * c.gid);
     tmem_ld8(t, v);
     tmem_ld8(t + kGC, w);
     tmem_ld_wait();
   #pragma unroll
     for (int i = 0; i < EC; ++i) v[i] += w[i];
     const int k = quarter * 32 + c.lane;
-    if (k < out_rows) epi(k, half, v);
+    if (k < out_rows) epi(k, v);
     tc_fence_before();
     }
-  if (!kIssuerFence) fence_proxy_async();
   c.phase ^= 1u;
   group_sync(c.gid);
 }
 
 // the same for a layer with at most 64 output rows whose weight rows are REPLICATED in the upper 64 lanes of the tensor-memory operand:
-// all eight warps of the group take part, lane quarters 0 / 1 on clips 0..3 of their 8-clip half, quarters 2 / 3 (the replicas) on
-// clips 4..7 -- four clips per thread instead of eight halves the dependent chain of the epilogue (the longest part of a layer)
+// all four warps of the group take part, lane quarters 0 / 1 on clips 0..3, quarters 2 / 3 (the replicas) on clips 4..7 -- four
+// clips per thread instead of eight halves the dependent chain of the epilogue (the longest part of a layer)
 template <int L, bool FWD, bool B_KMAJOR = false, class Epi>
 __device__ __forceinline__ void tc_layer4(Ctx& c, const unsigned char* src, int out_rows, Epi epi) {
   SmemT& S = *c.S;
   tc_issue<L, FWD, B_KMAJOR>(c, src);
-  const int quarter = c.wg & 3, half = c.wg >> 2, sub = quarter >> 1;
+  const int quarter = c.wg & 3, sub = quarter >> 1;
   if ((quarter & 1) * 32 < out_rows) {
     mbar_wait(&S.bar_mma[c.gid], c.phase);
     tc_fence_after();
     float v[4], w[4];
-    const uint32_t t = c.tmem + ((uint32_t)(quarter * 32) << 16) + kT_D + (uint32_t)(2 * kGC * c.gid + EC * half + 4 * sub);
+    const uint32_t t = c.tmem + ((uint32_t)(quarter * 32) << 16) + kT_D + (uint32_t)(2 * kGC * c.gid + 4 * sub);
     tmem_ld4(t, v);
     tmem_ld4(t + kGC, w);
     tmem_ld_wait();
 #pragma unroll
     for (int i = 0; i < 4; ++i) v[i] += w[i];
     const int k = (quarter & 1) * 32 + c.lane;
-    if (k < out_rows) epi(k, half, sub, v);
+    if (k < out_rows) epi(k, sub, v);
     tc_fence_before();
   }
-  if (!kIssuerFence) fence_proxy_async();
   c.phase ^= 1u;
   group_sync(c.gid);
 }
@@ -377,10 +359,9 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
   const P2 inv3e2 = mk2(inv3e[0], inv3e[1]), lrot9e2 = mk2(lrot9e[0], lrot9e[1]);
   __syncwarp();
   fence_proxy_async();
-  if (kKinGate && threadIdx.x < 2) S.kin_done[threadIdx.x] = 0;
   mbar_wait(&S.bar_w, 0);  // model image (biases, statistics, skeleton tables) has landed
   tc_fence_before();
-  __syncthreads();         // tensor-memory weights written by all warps; latent pieces and tracker rows of both groups in place
+  __syncthreads();         // tensor-memory weights written by all warps; latent pieces and tracker rows of every group in place
   tc_fence_after();
 
   const FkLaneIdx lane_idx = fk_lane_idx(M, lane);  // skeleton indices of this lane, in registers for the whole launch
@@ -388,25 +369,25 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
   const int slot0 = 2 * kG8 * gid;       // first 8-group (piece 1) of this group in the activation images
   unsigned neg0 = 0, neg1 = 0;           // LeakyReLU slope bits of (feature k, this thread's 4 clips) for the backward pass
   auto forward = [&]() {
-    tc_layer4<0, true>(ctx, S.ping, DP_H0, [&](int k, int half, int sub, float (&v)[4]) {
+    tc_layer4<0, true>(ctx, S.ping, DP_H0, [&](int k, int sub, float (&v)[4]) {
       const float b = M.b0[k];
       neg0 = 0;
 #pragma unroll
       for (int i = 0; i < 4; ++i) { v[i] = fmaf(v[i], wsc, b); neg0 |= (v[i] > 0.f ? 0u : 1u) << i; v[i] = lrelu(v[i]); }
-      store_pieces4(S.pong, k, slot0 + half, sub, v);
+      store_pieces4(S.pong, k, slot0, sub, v);
     });
-    tc_layer4<1, true>(ctx, S.pong, DP_H1, [&](int k, int half, int sub, float (&v)[4]) {
+    tc_layer4<1, true>(ctx, S.pong, DP_H1, [&](int k, int sub, float (&v)[4]) {
       const float b = M.b1[k];
       neg1 = 0;
 #pragma unroll
       for (int i = 0; i < 4; ++i) { v[i] = fmaf(v[i], wsc, b); neg1 |= (v[i] > 0.f ? 0u : 1u) << i; v[i] = lrelu(v[i]); }
-      store_pieces4(S.ping, k, slot0 + half, sub, v);
+      store_pieces4(S.ping, k, slot0, sub, v);
     });
-    tc_layer<2, true>(ctx, S.ping, DP_Y, [&](int k, int half, float (&v)[EC]) {
+    tc_layer<2, true>(ctx, S.ping, DP_Y, [&](int k, float (&v)[EC]) {
       const float b = M.b2[k];
 #pragma unroll
-      for (int i = 0; i < EC; i += 2)  // clips 2p, 2p + 1 of this 8-clip half = pair kGW gid + 4 half + p; feature k = 4 j + c
-        *reinterpret_cast<float2*>(reinterpret_cast<float*>(&S.y2[kGW * gid + 4 * half + i / 2][(k >> 1) & 1][k >> 2]) + 2 * (k & 1)) =
+      for (int i = 0; i < EC; i += 2)  // clips 2p, 2p + 1 of the group = pair kGW gid + p; feature k = 4 j + c
+        *reinterpret_cast<float2*>(reinterpret_cast<float*>(&S.y2[kGW * gid + i / 2][(k >> 1) & 1][k >> 2]) + 2 * (k & 1)) =
             make_float2(fmaf(v[i], wsc, b), fmaf(v[i + 1], wsc, b));
     });
   };
@@ -417,10 +398,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
   const float lt_scale = A.lambda_t * (1.0f / (float)DP_L);
   // A fixed number of iterations (negative stop thresholds, min_loss_incr = -inf: the headline workload) looks at the tracker losses
   // of an iteration only to report the last ones: their warp sums are skipped on the other iterations (dp_fk2.cuh, want_loss)
-#ifndef DP_LOSS_SKIP
-#define DP_LOSS_SKIP 1
-#endif
-  const bool fixed_iters = DP_LOSS_SKIP && A.eps_pos < 0.0 && A.eps_rot < 0.0 && A.min_incr < -1.7e308 && !A.trace && !A.eval_only;
+  const bool fixed_iters = A.eps_pos < 0.0 && A.eps_rot < 0.0 && A.min_incr < -1.7e308 && !A.trace && !A.eval_only;
   const bool clocked = CLOCK && A.phase_cycles != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
   long long tick = clocked ? clock64() : 0;
   auto phase_done = [&](int i) {
@@ -435,7 +413,6 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
   auto stamp = [&](int it, int k) {
     if (CLOCK && tl_on && it >= 40 && it < 44) A.phase_cycles[16 + gid * 24 + (it - 40) * 6 + k] = (unsigned long long)clock64();
   };
-  const bool gate_on = kKinGate && A.max_iter < (1 << 18);
   for (int it = 0; it < A.max_iter; ++it) {
     if (!group_or(gid, active[0] || active[1])) break;  // also publishes the latent pieces written by the Adam epilogue
     if (lane == 0) {  // the Adam epilogue reads two table entries: pull their lines into L1 now instead of stalling there
@@ -448,11 +425,6 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
     phase_done(0);
     stamp(it, 1);
     float nlp[CPW] = {0.f, 0.f}, nlr[CPW] = {0.f, 0.f};
-    if (kKinGate && gate_on) {  // wait for this team's turn (the counters only grow; a group that leaves the loop opens the gate for good)
-      const uint32_t need = 2u * (uint32_t)(it + (gid & 1));
-      const volatile uint32_t* other = &S.kin_done[(gid & 1) ^ 1];
-      while ((int32_t)(*other - need) < 0) {}
-    }
     if (active[0] || active[1]) {  // both clips of the warp in one packed pass; results of a stopped clip are discarded
       // one packed pass; dL/dy leaves it scaled per clip into [16, 32) (exact powers of two, undone when dL/dz is read)
       const FkOut2 o = fk_loss2<true, false, true>(M, lane_idx, &S.y2[warp][0][0], &S.trk2[warp][0][0], &S.groot2[warp][0], &S.fkscr[warp][0],
@@ -463,21 +435,19 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
       if (active[1]) { nlp[1] = o.lp.v.y; nlr[1] = o.lr.v.y; }
     }
     stamp(it, 2);
-    if (!kIssuerFence) fence_proxy_async();  // the dL/dy pieces are read by the tensor core (async proxy)
     group_sync(gid);
-    if (kKinGate && gate_on && wg == 0 && lane == 0) atomicAdd(&S.kin_done[gid & 1], 1u);
     phase_done(1);
     stamp(it, 3);
     // backward layers; dL/dy pieces were written by the kinematics warps (EmitDyPieces)
-    tc_layer4<2, false, true>(ctx, S.dyimg, DP_H1, [&](int k, int half, int sub, float (&v)[4]) {
+    tc_layer4<2, false, true>(ctx, S.dyimg, DP_H1, [&](int k, int sub, float (&v)[4]) {
 #pragma unroll
       for (int i = 0; i < 4; ++i) v[i] *= ((neg1 >> i) & 1u) ? 0.2f * wsc : wsc;
-      store_pieces4(S.ping, k, slot0 + half, sub, v);
+      store_pieces4(S.ping, k, slot0, sub, v);
     });
-    tc_layer4<1, false>(ctx, S.ping, DP_H0, [&](int k, int half, int sub, float (&v)[4]) {
+    tc_layer4<1, false>(ctx, S.ping, DP_H0, [&](int k, int sub, float (&v)[4]) {
 #pragma unroll
       for (int i = 0; i < 4; ++i) v[i] *= ((neg0 >> i) & 1u) ? 0.2f * wsc : wsc;
-      store_pieces4(S.pong, k, slot0 + half, sub, v);
+      store_pieces4(S.pong, k, slot0, sub, v);
     });
     phase_done(2);
     stamp(it, 4);
@@ -547,7 +517,6 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
       // EVERY clip (stopped and padding clips included) so that no column ever feeds back on its own garbage -- a
       // non-finite value in a K-padding row would poison the column through 0 x NaN
       if (lat) store_piece_pair(S.ping, lane, gid, 2 * wg, z.x, z.y);
-      if (!kIssuerFence) fence_proxy_async();
       // early-stop bookkeeping: every lane holds the same (warp-uniform) numbers
       const float total0 = (nlp[0] + nlr[0]) + nlt0, total1 = (nlp[1] + nlr[1]) + nlt1;
       const double incr0 = prev0 - (double)total0, incr1 = prev1 - (double)total1;
@@ -570,14 +539,12 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
     stamp(it, 5);
   }
 
-  if (kKinGate && gate_on && wg == 0 && lane == 0) atomicAdd(&S.kin_done[gid & 1], 1u << 20);  // out of the loop: never make the other team wait again
   // ---- frame epilogue (drag_pose.py:369-414) from the LAST EVALUATED latent (pre-step)
   __syncwarp();
   if (lane < DP_L) {
     const float2 zl = S.st[warp][ST_ZLAST][lane];
     store_piece_pair(S.ping, lane, gid, 2 * wg, zl.x, zl.y);
   }
-  if (!kIssuerFence) fence_proxy_async();
   group_sync(gid);
   forward();
   P2 q2[4], r2[4], p2[3], d2[3];
@@ -659,7 +626,7 @@ cudaError_t dp_frame_tc16_launch(const DpFrameArgs& args, int num_sms, cudaStrea
   if (cudaError_t e = clk ? dp_ensure_smem(dp_frame_tc16_kernel<true>, smem, configured_clk) : dp_ensure_smem(dp_frame_tc16_kernel<false>, smem, configured);
       e != cudaSuccess)
     return e;
-  // spread the clips over every SM: 4096 clips -> 28 per CTA (two groups of 14) on 147 SMs
+  // spread the clips over every SM: 4096 clips -> 28 per CTA (14 pairs dealt 4 + 4 + 3 + 3 to the groups) on 147 SMs
   DpFrameArgs a = args;
   int cpc = (args.n_clips + num_sms - 1) / num_sms;
   cpc = cpc < 1 ? 1 : (cpc > NC ? NC : cpc);

@@ -20,8 +20,6 @@ inline cudaError_t dp_ensure_smem(Kernel kernel, size_t smem, std::atomic<unsign
   return e;
 }
 
-#define DP_PRED_MAX_PARTS 4
-#define DP_PRED_PARTS_DEFAULT 2
 struct TpWork {
   float* enc;
   float* enc2;
@@ -30,8 +28,8 @@ struct TpWork {
   float* dec_lat;
   float* ffpart; // hidden-split partial sums of the feed-forward kernel (DP_FF_PART_FLOATS)
   int num_sms;
-  cudaStream_t st_extra[DP_PRED_MAX_PARTS - 1];  // extra streams + fork/join events: the predictor of a large batch runs in parts
-  cudaEvent_t ev_fork, ev_join[DP_PRED_MAX_PARTS - 1];
+  cudaStream_t st_extra;  // second stream + fork/join events: the predictor of a large batch runs in two parts
+  cudaEvent_t ev_fork, ev_join;
   struct TpGraphCache* graphs;  // replayable launch chains of small predictor calls (dp_temporal.cu); null = always launch kernel by kernel
 };
 // A small predictor call (B = 1 streaming: ~70 kernels of a few microseconds each at window 16) is bound by launch gaps, not by work.

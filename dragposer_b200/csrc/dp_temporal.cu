@@ -545,13 +545,9 @@ static cudaError_t run_part(const float* blob, const TpLayout& L, const float* m
     }
     *launches += 2;
   }
-#ifdef DP_DEBUG_SKIP_DEC  // measurement only (wrong targets): how much of a call is the decoder?
-  if (B > 1024) return cudaGetLastError();
-#endif
   int T = 1;
-  static const int fused_dec = getenv("DP_PRED_FUSED_DEC") ? atoi(getenv("DP_PRED_FUSED_DEC")) : 1;
   for (int i = 0; i <= window; i += 4, ++T) {
-    if (fftiles && fused_dec && T == 1 && (size_t)4 * B * TP_D <= part_floats) {
+    if (fftiles && T == 1 && (size_t)4 * B * TP_D <= part_floats) {
       // single-token pass: embedding + self- and cross-attention of layer 0 in one small kernel, then per layer the feed-forward block
       // with the next layer's two attention blocks (or the prediction head) fused into its finishing kernel: 7 launches, none of them
       // an attention kernel (round 2 started at 17, then 10 with tcgen05 cross-attention launches)
@@ -664,9 +660,14 @@ void dp_temporal_graphs_destroy(TpGraphCache* c) {
   delete c;
 }
 
-// The predictor of a large batch runs as several parts on their own streams: each kernel of a part has fewer tiles than the device has
-// CTA slots, so the block scheduler interleaves the parts and fills the tail of one kernel with the head of another
-// (448 tiles on 296 slots otherwise leave a third, half-empty round in every encoder kernel).
+// The predictor of a batch of kPredSplitMin or more virtual clips runs as two parts on two streams: each kernel of a part has fewer
+// tiles than the device has CTA slots, so the block scheduler interleaves the parts and fills the tail of one kernel with the head of
+// the other (448 tiles on 296 slots otherwise leave a third, half-empty round in every encoder kernel).  Two parts measured faster
+// than one or four (DESIGN.md section 3.2).
+constexpr int kPredSplitMin = 2048;
+// Hidden-split workspace of one part: a quarter of DP_FF_PART_FLOATS, not a half.  dp_ff_tc_launch picks the split from it, and with
+// a half the decoder feed-forward of an 8 192-virtual-clip part would be split 8-fold instead of 4-fold: another summation order.
+constexpr size_t kPredPartFloats = DP_FF_PART_FLOATS / 4;
 cudaError_t dp_temporal_run(const float* blob, const TpLayout& L, const float* mu, const float* sigma,
                             const float* latent_buf, const float* disp_buf, const float* height_buf, int head, int n_real,
                             int window, float* target_buf, const TpWork& w, const unsigned char* fftiles, cudaStream_t st,
@@ -674,12 +675,9 @@ cudaError_t dp_temporal_run(const float* blob, const TpLayout& L, const float* m
   const int B = n_real * J;  // virtual clips
   cudaError_t err = cudaFuncSetAttribute(tp_ff_ln_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFfSmem);
   if (err != cudaSuccess) return err;
-  static const int split_min = getenv("DP_PRED_SPLIT_MIN") ? atoi(getenv("DP_PRED_SPLIT_MIN")) : 2048;
-  static const int n_parts_env = getenv("DP_PRED_PARTS") ? atoi(getenv("DP_PRED_PARTS")) : DP_PRED_PARTS_DEFAULT;
-  const int n_parts = n_parts_env < 1 ? 1 : (n_parts_env > DP_PRED_MAX_PARTS ? DP_PRED_MAX_PARTS : n_parts_env);
-  if (!fftiles || n_parts == 1 || B < split_min) {
-    // DP_PRED_GRAPH=0 turns the replay off; the pipeline-clock switches synchronise inside a launch function, which a capture forbids
-    static const int use_graphs = (getenv("DP_PRED_GRAPH") ? atoi(getenv("DP_PRED_GRAPH")) : 1) && !getenv("DP_FF_TRACE") && !getenv("DP_ATTN_TRACE");
+  if (!fftiles || B < kPredSplitMin) {
+    // no replay while a pipeline clock is on: DP_FF_TRACE / DP_ATTN_TRACE synchronise inside a launch function, which a capture forbids
+    static const bool use_graphs = !getenv("DP_FF_TRACE") && !getenv("DP_ATTN_TRACE");
     auto eager = [&](int stage) {
       return run_part(blob, L, mu, sigma, latent_buf, disp_buf, height_buf, head, B, 0, J, window, target_buf, w, DP_FF_PART_FLOATS, fftiles, st, launches, stage);
     };
@@ -718,28 +716,22 @@ cudaError_t dp_temporal_run(const float* blob, const TpLayout& L, const float* m
     return cudaSuccess;
   }
   if ((err = cudaEventRecord(w.ev_fork, st)) != cudaSuccess) return err;
-  static const int part_clips_env = getenv("DP_PRED_PART_CLIPS") ? atoi(getenv("DP_PRED_PART_CLIPS")) : 0;
-  int per = (B + n_parts - 1) / n_parts, parts = n_parts;
-  if (part_clips_env > 0 && (B + part_clips_env - 1) / part_clips_env <= DP_PRED_MAX_PARTS) {
-    per = part_clips_env;
-    parts = (B + per - 1) / per;
-  }
-  for (int p = 0; p < parts; ++p) {
-    const int b0 = p * per, nb = (b0 + per <= B ? per : B - b0);
-    if (nb <= 0) break;
-    cudaStream_t sp = p == 0 ? st : w.st_extra[p - 1];
+  const int per = (B + 1) / 2;
+  for (int p = 0; p < 2; ++p) {
+    const int b0 = p * per, nb = p == 0 ? per : B - per;
+    cudaStream_t sp = p == 0 ? st : w.st_extra;
     if (p > 0 && (err = cudaStreamWaitEvent(sp, w.ev_fork, 0)) != cudaSuccess) return err;
     TpWork wp = w;
     wp.enc += (size_t)b0 * TP_S * TP_D; wp.enc2 += (size_t)b0 * TP_S * TP_D;
     wp.dec += (size_t)b0 * TP_MAXT * TP_D; wp.dec2 += (size_t)b0 * TP_MAXT * TP_D;
     wp.dec_lat += (size_t)b0 * TP_MAXT * TP_LAT;
-    wp.ffpart += (DP_FF_PART_FLOATS / DP_PRED_MAX_PARTS) * p;
+    wp.ffpart += kPredPartFloats * p;
     err = run_part(blob, L, mu, sigma, latent_buf, disp_buf, height_buf, head, nb, b0, J, window, target_buf + (size_t)b0 * (window + 1) * TP_LAT, wp,
-                   DP_FF_PART_FLOATS / DP_PRED_MAX_PARTS, fftiles, sp, launches);
+                   kPredPartFloats, fftiles, sp, launches);
     if (err != cudaSuccess) return err;
     if (p > 0) {
-      if ((err = cudaEventRecord(w.ev_join[p - 1], sp)) != cudaSuccess) return err;
-      if ((err = cudaStreamWaitEvent(st, w.ev_join[p - 1], 0)) != cudaSuccess) return err;
+      if ((err = cudaEventRecord(w.ev_join, sp)) != cudaSuccess) return err;
+      if ((err = cudaStreamWaitEvent(st, w.ev_join, 0)) != cudaSuccess) return err;
     }
   }
   return cudaSuccess;

@@ -19,18 +19,10 @@
 #define TP_PE 30
 #define TP_NENC 3
 #define TP_NDEC 3
-#ifndef DP_FF_QUAD
-#define DP_FF_QUAD 1              // 1 (default): the feed-forward kernel re-tiled for four CTAs per SM (dp_temporal_tc4.cuh); 0: two CTAs per SM (dp_temporal_tc.cuh)
-#endif
-#if DP_FF_QUAD
+// weight image of the tensor-core feed-forward block (dp_temporal_tc4.cuh)
 #define FFT_HC 32                 // hidden units per tensor-core FF chunk
 #define FFT_STEP_BYTES 12288      // one pipeline step: W2c pieces of chunk t-1 (2 x 3072 fp16) + W1c pieces of chunk t (2 x 3072 fp16)
 #define FFT_LAYER_BYTES (TP_FF * 4 + (TP_FF / FFT_HC + 1) * FFT_STEP_BYTES)   // b1 (fp32) + 65 steps
-#else
-#define FFT_HC 64                 // hidden units per tensor-core FF chunk
-#define FFT_STEP_BYTES 24576      // one pipeline step: W2c pieces of chunk t-2 (2 x 6144 fp16) + W1c pieces of chunk t (2 x 6144 fp16)
-#define FFT_LAYER_BYTES (TP_FF * 4 + (TP_FF / FFT_HC + 2) * FFT_STEP_BYTES)   // b1 (fp32) + 34 steps
-#endif
 #define ATT_LAYER_BYTES 37632      // W_in pieces (2 x 13824 fp16) + W_o pieces (2 x 4608 fp16) + b_in (576) + b_o (192)
 
 struct TpAttn {   // offsets (floats) into the blob

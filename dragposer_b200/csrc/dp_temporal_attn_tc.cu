@@ -1,5 +1,5 @@
-// dp_temporal_attn_tc.cu -- stand-alone launches of the tensor-core attention block (dp_temporal_attn_tc.cuh): decoder self- and
-// cross-attention, and the encoder self-attention when the fused encoder kernel (dp_temporal_enc_tc.cu) is not used.
+// dp_temporal_attn_tc.cu -- launches of the tensor-core attention block (dp_temporal_attn_tc.cuh): encoder self-attention and
+// decoder self- and cross-attention.
 #include <cuda_fp16.h>
 
 #include <cstdio>

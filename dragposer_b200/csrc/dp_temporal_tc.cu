@@ -1,5 +1,5 @@
-// dp_temporal_tc.cu -- stand-alone launches of the tensor-core feed-forward block (dp_temporal_tc.cuh): every decoder layer, and
-// the encoder layers when the fused encoder kernel (dp_temporal_enc_tc.cu) is not used.
+// dp_temporal_tc.cu -- launches of the tensor-core feed-forward block (dp_temporal_tc4.cuh) for every encoder and decoder layer,
+// the finishing kernels of its hidden-split mode, and the host-side packing of its weight image.
 #include <cuda_fp16.h>
 
 #include <cstdio>
@@ -7,11 +7,7 @@
 #include <cstring>
 
 #include "dp_temporal.cuh"
-#if DP_FF_QUAD
 #include "dp_temporal_tc4.cuh"
-#else
-#include "dp_temporal_tc.cuh"
-#endif
 
 using namespace tpf;
 
@@ -151,7 +147,7 @@ void dp_ff_tc_pack(const float* w1t, const float* b1, const float* w2t, unsigned
           r -= __half2float(w1p[p][off]);
         }
       }
-    // W2c as B operand [N = out 48][K = hidden chunk] -> first half of step c + 2
+    // W2c as B operand [N = out 48][K = hidden chunk] -> first half of step c + kLag
     __half* w2p[2] = {reinterpret_cast<__half*>(steps + (size_t)(c + kLag) * kStepBytes),
                       reinterpret_cast<__half*>(steps + (size_t)(c + kLag) * kStepBytes + kW2Bytes)};
     for (int n = 0; n < TP_D; ++n)
@@ -173,9 +169,9 @@ cudaError_t dp_ff_tc_launch(const unsigned char* wimg, const float* blob, const 
   const size_t smem = sizeof(Smem) + 1024;
   if (cudaError_t e = dp_ensure_smem(tp_ff_tc_kernel, smem, configured); e != cudaSuccess) return e;
   const int tiles = (n_rows + kTM - 1) / kTM;
-  // hidden split: largest power of two that still leaves every CTA resident at once (two CTAs per SM) and >= 4 chunks each
+  // hidden split: largest power of two that still leaves every CTA resident at once (kCtasPerSm per SM) and >= 4 chunks each
   int n_split = 1;
-  constexpr int kMaxSplit = kChunks / 4;  // at least four chunks per CTA: 8 with 64-unit chunks, 16 with 32-unit chunks
+  constexpr int kMaxSplit = kChunks / 4;  // at least four chunks per CTA: 16
   while (n_split < kMaxSplit && tiles * n_split * 2 <= kCtasPerSm * num_sms && (size_t)(n_split * 2) * n_rows * TP_D <= part_floats) n_split *= 2;
   if (!part) n_split = 1;
   if (tail) {  // the tail runs in the finish kernel: keep the split path even for a batch that would fill the device unsplit

@@ -1,11 +1,20 @@
 #pragma once
-// dp_temporal_tc4.cuh -- the feed-forward block of dp_temporal_tc.cuh re-tiled for FOUR CTAs per SM (-DDP_FF_QUAD=1).
+// dp_temporal_tc4.cuh -- feed-forward block of the temporal predictor on tcgen05 tensor cores, four CTAs per SM.
 //
-// The pipeline clock of the two-CTA kernel (profiles/r2_ff_pipeline_clock.md) shows a tile saturating the tensor pipe inside its
-// chunks and losing a third of its time around them (the L2 fill burst of a wave at its start, the row epilogue at its end), in
-// phase on both CTAs of an SM.  Here a CTA is half the size in every resource -- 128 tensor-memory columns (ONE 32-unit H buffer that
-// the pieces overwrite in place), a 3 x 12 KB weight ring, four epilogue warps -- so four of them share an SM and its tensor pipe:
-// while one is starting or finishing, three are multiplying.
+//   out = LayerNorm(x + W2 relu(W1 x + b1) + b2)   [+ optional second LayerNorm]
+// (torch nn.TransformerEncoderLayer / DecoderLayer FF sub-block, post-norm, d_model 48, dim_feedforward 2048;
+// python/src/temporal_transformer.py:26-33): 95% of the predictor's FLOPs.  One CTA owns a tile of 128 tokens (the UMMA M
+// dimension) and walks the 2048 hidden units in chunks of 32.  Precision: fp16x2 split products on kind::f16 -- every fp32 value
+// is two fp16 pieces, three products (2,1)(1,2)(1,1) accumulate in fp32; the weight image stores 64 W (an exact power of two,
+// undone in the epilogues) so that the second piece of the small FF weights stays a normal fp16.  A operands live in tensor memory
+// (TS mode): X is split once into TMEM and the epilogue warps write the packed pieces of relu(H) over the accumulator they came
+// from, so activations never touch shared memory.  Weights are pre-split and pre-tiled on the host (dp_ff_tc_pack) into the exact
+// shared-memory operand image: one pipeline step is ONE bulk-TMA copy, fed by a producer warp to an issuer warp through a
+// mbarrier ring.
+// A CTA is small in every resource -- 128 tensor-memory columns (ONE 32-unit H buffer that the pieces overwrite in place), a
+// 3 x 12 KB weight ring, four epilogue warps -- so four of them share an SM and its tensor pipe: a tile saturates the pipe inside
+// its chunks and loses time around them (the L2 fill burst of a wave at its start, the row epilogue at its end,
+// profiles/r2_ff_pipeline_clock.md), and while one CTA is starting or finishing, three are multiplying.
 //   MMA1  H[128x32]  = X[128x48] . W1c^T     (K = 48, 9 MMAs)
 //   epi   H -> +b1, relu, split -> the same 32 columns (two packed pieces of 16 words)
 //   MMA2  O[128x48] += H[128x32] . W2c^T     (K = 32, 6 MMAs)
@@ -93,7 +102,11 @@ __device__ __forceinline__ void ff_init_barriers(Smem& S) {
   mbar_init(&S.hready, kEpiThreads);
   mbar_init(&S.b1full, 1);
 }
-// Same contract as ff_tile of dp_temporal_tc.cuh (one 128-row tile, hidden split (split, n_split), raw partial sums to `part` when split).
+// One feed-forward block for the 128-row tile starting at row0 (rows >= m_limit of the tile are padding).  (split, n_split): this
+// call takes the hidden chunks [split, split + 1) * kChunks / n_split; with n_split > 1 the raw partial sums go to `part`
+// ([n_split][n_rows][48]) and tp_ff_finish_kernel adds bias, residual and the LayerNorms.  Called by all kThreads threads with
+// kT_COLS columns of tensor memory at `tmem` and the mbarriers of S freshly initialised and published by a block barrier; returns
+// after a block barrier.
 __device__ __forceinline__ void ff_tile(Smem& S, const uint32_t tmem, const unsigned char* wimg, const float* blob, TpFF F, TpNorm N1, TpNorm N2, int has_n2,
                                         const float* x_g, int n_rows, int T, int row_stride, int row0, int m_limit, int split, int n_split,
                                         float* out_g, float* part, long long* trace) {
@@ -180,7 +193,9 @@ __device__ __forceinline__ void ff_tile(Smem& S, const uint32_t tmem, const unsi
       tmem_ld32(tmem + lane_base + kT_H, v);
       tmem_ld_wait();
       if (traced && i < 32) trace[i * 8 + 5] = clock64();
-      // three CUDA-core instructions per hidden unit (see dp_temporal_tc.cuh): p1 = relu(h) rounded towards zero, p2 = relu(h - p1)
+      // three CUDA-core instructions per hidden unit: packed FFMA2 for scale + bias and FADD2 for the residual, the ReLU folded into
+      // the conversions.  Piece 1 is relu(h) rounded TOWARDS ZERO (cvt.rz.relu), so the residual h - p1 of a positive h is never
+      // negative, while a negative h (p1 = 0) leaves a negative residual that piece 2's cvt.rn.relu clamps: p1 + p2 = relu(h) to 2^-21
 #pragma unroll
       for (int j = 0; j < 32; j += 2) {
         const float2 h = __ffma2_rn(make_float2(v[j], v[j + 1]), make_float2(1.0f / kFfWScale, 1.0f / kFfWScale), make_float2(b1[j], b1[j + 1]));

@@ -18,6 +18,6 @@ ts = np.zeros(T)
 for t in range(T):
     t0 = time.perf_counter(); eng.run(wl["tgt_pos"][t], wl["tgt_rot"][t], wl["joints"], wl["weights"], **kw); ts[t] = time.perf_counter() - t0
 ts = ts[64:].reshape(-1, 16)
-print("DP_PRED_PREFETCH=%s DP_PRED_GRAPH=%s  median call time (us) by window index:" % (os.environ.get("DP_PRED_PREFETCH", "1"), os.environ.get("DP_PRED_GRAPH", "1")))
+print("DP_PRED_PREFETCH=%s  median call time (us) by window index:" % os.environ.get("DP_PRED_PREFETCH", "1"))
 print(" ".join(f"{1e6 * v:.0f}" for v in np.median(ts, axis=0)), f"| mean {1e6 * ts.mean():.1f}")
 eng.close()

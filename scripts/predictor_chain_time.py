@@ -1,5 +1,5 @@
-"""B = 1 predictor call at window 16 (5 decoder passes, ~70 kernels): wall time of dp_engine_predict_targets + device synchronisation,
-kernel by kernel (DP_PRED_GRAPH=0) or as a replayed CUDA graph (default).  Run once per setting: the switch is read once per process."""
+"""B = 1 predictor call at window 16 (5 decoder passes, ~70 kernels): wall time of dp_engine_predict_targets + device synchronisation.
+From the second call of a shape on, everything after the embedding kernel is a replayed CUDA graph; the first five calls are not counted."""
 import os, sys, time
 import numpy as np
 import torch
@@ -23,6 +23,6 @@ for W in (16, 0):
         t1 = time.perf_counter()
         torch.cuda.synchronize()
         ts.append(time.perf_counter() - t0); te.append(t1 - t0)
-    print(f"{B} clip(s), window {W}, DP_PRED_GRAPH={os.environ.get('DP_PRED_GRAPH', '1')}: enqueue p50 {1e6 * np.median(te[5:]):.0f} us, "
+    print(f"{B} clip(s), window {W}: enqueue p50 {1e6 * np.median(te[5:]):.0f} us, "
           f"enqueue + device p50 {1e6 * np.median(ts[5:]):.0f} us")
 eng.close()

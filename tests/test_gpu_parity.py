@@ -365,8 +365,8 @@ def test_tcgen05_paths_agree_with_cuda_core_path_multi_wave(engine_factory, pose
 @pytest.mark.parametrize("n_clips", [1, 37, 300, 2101, 8200])
 def test_temporal_predictor_tensor_core_vs_cuda_core(golden_dir, engine_factory, n_clips):
     """Every decoder length (T = 1 + W/4 up to 30 tokens), ragged last tiles, a batch large enough (>= 2048 clips) to run the
-    predictor as two parts on two streams, and one (8200 clips: 449 row tiles per part on 296 resident CTAs) whose persistent
-    feed-forward CTAs walk two tiles each, the second one ragged for some: tcgen05 kernels vs the fp32 CUDA-core kernels."""
+    predictor as two parts on two streams, and one (8200 clips: 449 encoder row tiles per part, the last one ragged) large enough
+    that the encoder feed-forward runs without the hidden split: tcgen05 kernels vs the fp32 CUDA-core kernels."""
     g = np.load(os.path.join(golden_dir, "ref_temporal.npz"))
     rng = np.random.default_rng(5)
     reps = -(-n_clips // g["latent_buf"].shape[0])
