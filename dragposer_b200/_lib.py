@@ -81,6 +81,9 @@ SIGNATURES = {
     "dp_engine_get_phase_cycles": (C.c_int, [_VP, C.POINTER(C.c_ulonglong)]),
     "dp_engine_get_timeline": (C.c_int, [_VP, C.POINTER(C.c_ulonglong)]),
     "dp_engine_get_profile": (C.c_int, [_VP, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),
+    "dp_engine_restart_clips": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "dp_engine_get_clip_index": (C.c_int, [_VP, C.c_int, _VP]),
+    "dp_engine_frames_to_boundary": (C.c_int, [_VP, C.c_int]),
 }
 
 _lib = None

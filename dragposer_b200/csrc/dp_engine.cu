@@ -7,6 +7,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <chrono>
@@ -91,6 +92,21 @@ struct dp_engine {
   int profiling = 0;
   unsigned long long* d_phase = nullptr;  // 8 phase-cycle counters + 48 timeline stamps of the tcgen05 frame kernel (profiling level 2 only)
   std::vector<cudaEvent_t> prof_events;  // triples: before predictor, before frame kernel, after frame kernel
+  // Per-clip restarts (dp_engine_restart_clips).  Clip c runs at its own predictor phase phase[c]: its own temporal index is
+  // (current_index - phase[c]) mod window, and its own target row k < window lives in slot (k + phase[c]) % window of d_target_buf
+  // (row window in slot window), so the frame kernels read slot current_index of every clip as before.  While every clip shares one
+  // phase it is folded into current_index (all phases 0, n_phases 1) and nothing differs from a batch that was never restarted.
+  std::vector<int> phase;        // (max_clips)
+  int n_phases = 1;              // distinct phases among the clips; >= 2 = mixed
+  std::vector<int> class_start;  // mixed phases: the clips of phase s are d_class[class_start[s] .. class_start[s + 1])
+  int32_t* d_class = nullptr;    // clip ids grouped by phase, ascending within a phase
+  // pinned staging of a restart: restarted ids (max_clips) | ids grouped by phase (max_clips) | state rows (max_clips, DP_RESTART_STATE);
+  // ev_restart follows its copies, so the next restart does not overwrite a block still in flight
+  unsigned char *h_restart = nullptr, *d_restart = nullptr;
+  cudaEvent_t ev_restart = nullptr;
+  bool restart_pending = false;
+  // compact inputs and outputs of the subset predictor (allocated on first use, max_clips rows)
+  float *d_sub_latent = nullptr, *d_sub_disp = nullptr, *d_sub_height = nullptr, *d_sub_target = nullptr;
 };
 
 extern "C" const char* dp_engine_last_error(void) { return g_err.c_str(); }
@@ -157,6 +173,8 @@ extern "C" int dp_engine_create(dp_engine** out, int device, int max_clips) {
   CK(cudaEventCreateWithFlags(&e->tw.ev_fork, cudaEventDisableTiming));
   CK(cudaStreamCreateWithFlags(&e->tw.st_extra, cudaStreamNonBlocking));
   CK(cudaEventCreateWithFlags(&e->tw.ev_join, cudaEventDisableTiming));
+  e->phase.assign(B, 0);
+  e->class_start.assign(DP_MAX_WINDOW + 2, 0);
   *out = e;
   return DP_OK;
 }
@@ -190,6 +208,9 @@ extern "C" int dp_engine_destroy(dp_engine* e) {
   if (e->ev_pre_fork) cudaEventDestroy(e->ev_pre_fork);
   if (e->ev_pre_done) cudaEventDestroy(e->ev_pre_done);
   cudaFree(e->d_target_alt);
+  cudaFreeHost(e->h_restart); cudaFree(e->d_restart);
+  if (e->ev_restart) cudaEventDestroy(e->ev_restart);
+  cudaFree(e->d_sub_latent); cudaFree(e->d_sub_disp); cudaFree(e->d_sub_height); cudaFree(e->d_sub_target);
   dp_temporal_graphs_destroy(e->tw.graphs);
   cudaStreamDestroy(e->stream);
   delete e;
@@ -384,6 +405,8 @@ extern "C" int dp_engine_init_clips(dp_engine* e, int n, const float* latent0, c
   e->target_rows = 0;
   e->look_left = 0;
   e->look_last_row = -1;
+  std::fill(e->phase.begin(), e->phase.end(), 0);
+  e->n_phases = 1;
   return DP_OK;
 }
 
@@ -446,11 +469,41 @@ static int check_n_ee(const int32_t* n_ee, size_t count, int ee_stride, const dp
   return DP_OK;
 }
 
+static int ensure_subset_scratch(dp_engine* e) {
+  if (e->d_sub_target) return DP_OK;
+  const size_t B = (size_t)e->max_clips;
+  CK(cudaMalloc(&e->d_sub_latent, B * DP_PAST * DP_L * 4));
+  CK(cudaMalloc(&e->d_sub_disp, B * DP_PAST * 3 * 4));
+  CK(cudaMalloc(&e->d_sub_height, B * DP_PAST * DP_NH * 4));
+  CK(cudaMalloc(&e->d_sub_target, B * (DP_MAX_WINDOW + 1) * DP_L * 4));
+  return DP_OK;
+}
+
+// The predictor for the n clips listed at d_ids (device) alone: their ring rows are gathered into compact buffers (same ring head),
+// the unmodified predictor runs on those, and its (n, window + 1, 24) rows are scattered into rows [r0, dst_rows) of dst -- rotated
+// by `shift` (see dp_engine::phase), or broadcast when window is 0.
+static int predict_subset(dp_engine* e, const int32_t* d_ids, int n, int window, float* dst, int dst_rows, int r0, int shift,
+                          cudaStream_t st) {
+  int rc = ensure_subset_scratch(e);
+  if (rc) return rc;
+  drop_prefetch(e);  // the predictor's work buffers
+  CK(dp_gather_rings_launch(d_ids, n, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, e->d_sub_latent, e->d_sub_disp, e->d_sub_height, st));
+  ++e->launches;
+  CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_sub_latent, e->d_sub_disp, e->d_sub_height, e->ring_head, n, window,
+                     e->d_sub_target, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles, st, &e->launches));
+  CK(dp_scatter_targets_launch(e->d_sub_target, window + 1, d_ids, n, dst, dst_rows, r0, window, shift, st));
+  ++e->launches;
+  return DP_OK;
+}
+
 static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, const int32_t* joints, const float* weights,
                    int shared, const float* tgt_pos, const float* tgt_rot, int ee_stride, float* out_pose, float* out_gpos,
                    cudaStream_t st) {
   const int W = p->temporal_future_window;
   if (e->target_rows != W + 1) {  // drag_pose.py:237-244: fresh zero buffer when the window changes
+    if (e->n_phases > 1)
+      return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own predictor phase: "
+                                "re-initialise the clips (dp_engine_init_clips) to change it");
     drop_prefetch(e);
     CK(cudaMemsetAsync(e->d_target_buf, 0, (size_t)e->n_clips * (W + 1) * DP_L * 4, st));
     e->target_rows = W + 1;
@@ -467,7 +520,14 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
   if (!look) {
     e->look_left = 0;
     e->look_last_row = -1;
-    if (e->current_index == 0) {
+    if (e->n_phases > 1) {  // mixed phases: the clips whose own frame 0 this is get their targets, the others keep theirs
+      const int s = e->current_index, n = e->class_start[s + 1] - e->class_start[s];
+      if (n > 0) {
+        if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
+        const int rc = predict_subset(e, e->d_class + e->class_start[s], n, W, e->d_target_buf, W + 1, 0, s, st);
+        if (rc) return rc;
+      }
+    } else if (e->current_index == 0) {
       if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
       if (e->pre_valid && e->pre_window == W) {  // issued three frames ago into the other buffer
         CK(cudaStreamWaitEvent(st, e->ev_pre_done, 0));
@@ -908,6 +968,15 @@ extern "C" int dp_engine_get_state(dp_engine* e, float* latent, float* gpos, flo
                       cudaMemcpyDeviceToHost));
     else
       CK(cudaMemcpy(target_buf, e->d_target_buf, B * e->target_rows * DP_L * 4, cudaMemcpyDeviceToHost));
+    if (e->n_phases > 1 && e->look_last_row < 0) {  // rotated rows (dp_engine::phase) -> each clip's own row order
+      const int W = e->target_rows - 1;
+      std::vector<float> own((size_t)W * DP_L);
+      for (size_t c = 0; c < B; ++c) {
+        float* rows = target_buf + c * e->target_rows * DP_L;
+        for (int k = 0; k < W; ++k) memcpy(&own[(size_t)k * DP_L], rows + (size_t)((k + e->phase[c]) % W) * DP_L, DP_L * 4);
+        memcpy(rows, own.data(), own.size() * 4);
+      }
+    }
   }
   if (current_index) *current_index = e->current_index;
   return DP_OK;
@@ -933,6 +1002,8 @@ extern "C" int dp_engine_predict_targets(dp_engine* e, int window, void* stream)
   if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
   if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
   if (window < 0 || window > DP_MAX_WINDOW || window % 4) return fail(DP_ERR_ARG, "window must be a multiple of 4 in [0,116]");
+  if (e->n_phases > 1)
+    return fail(DP_ERR_STATE, "dp_engine_predict_targets: restarted clips run at their own predictor phase (it predicts every clip at once)");
   CK(cudaSetDevice(e->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
   drop_prefetch(e);  // this call uses the predictor's work buffers
@@ -1004,3 +1075,106 @@ extern "C" int dp_engine_set_predictor_path(dp_engine* e, int path) {
 }
 
 extern "C" int dp_engine_last_decoder_path(const dp_engine* e) { return e ? e->last_path : 0; }
+
+extern "C" int dp_engine_restart_clips(dp_engine* e, int n, const int32_t* clips, const float* latent0, const float* gpos,
+                                       const float* grot, const float* heights, void* stream) {
+  if (!e || !clips || !latent0 || !gpos || !grot || !heights) return fail(DP_ERR_ARG, "dp_engine_restart_clips: null argument");
+  if (e->n_clips <= 0) return fail(DP_ERR_STATE, "dp_engine_restart_clips: no clips initialised (dp_engine_init_clips)");
+  if (n < 1 || n > e->n_clips) return fail(DP_ERR_ARG, "dp_engine_restart_clips: n out of range");
+  const int B = e->n_clips;
+  std::vector<char> seen(B, 0);
+  for (int i = 0; i < n; ++i) {
+    if (clips[i] < 0 || clips[i] >= B) return fail(DP_ERR_ARG, "dp_engine_restart_clips: clip id out of range");
+    if (seen[clips[i]]) return fail(DP_ERR_ARG, "dp_engine_restart_clips: duplicate clip id");
+    seen[clips[i]] = 1;
+  }
+  CK(cudaSetDevice(e->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+  const size_t cap = (size_t)e->max_clips;
+  if (!e->h_restart) {
+    const size_t bytes = cap * (8 + DP_RESTART_STATE * 4);
+    CK(cudaMallocHost(&e->h_restart, bytes));
+    CK(cudaMalloc(&e->d_restart, bytes));
+    CK(cudaEventCreateWithFlags(&e->ev_restart, cudaEventDisableTiming));
+    e->d_class = reinterpret_cast<int32_t*>(e->d_restart + cap * 4);
+  }
+  if (e->restart_pending) CK(cudaEventSynchronize(e->ev_restart));  // the previous restart's copies have left the pinned block
+  e->restart_pending = false;
+  drop_prefetch(e);  // targets computed ahead from the restarted clips' old rows are void
+  // Each restarted clip's next frame is its own frame 0, i.e. its phase is the index the next frame runs at.
+  const int W = e->target_rows > 1 ? e->target_rows - 1 : 0;
+  const int g = e->current_index;
+  std::vector<int> phase(e->phase.begin(), e->phase.begin() + B);
+  for (int i = 0; i < n; ++i) phase[clips[i]] = g;
+  std::vector<int> count(DP_MAX_WINDOW + 1, 0);
+  int distinct = 0;
+  for (int c = 0; c < B; ++c) distinct += count[phase[c]]++ == 0;
+  int32_t* h_ids = reinterpret_cast<int32_t*>(e->h_restart);
+  int32_t* h_class = h_ids + cap;
+  float* h_state = reinterpret_cast<float*>(e->h_restart + cap * 8);
+  memcpy(h_ids, clips, (size_t)n * 4);
+  for (int i = 0; i < n; ++i) {
+    float* s = h_state + (size_t)i * DP_RESTART_STATE;
+    memcpy(s, latent0 + (size_t)i * DP_L, DP_L * 4);
+    memcpy(s + DP_L, gpos + (size_t)i * 3, 12);
+    memcpy(s + DP_L + 3, grot + (size_t)i * 4, 16);
+    memcpy(s + DP_L + 7, heights + (size_t)i * DP_NH, DP_NH * 4);
+  }
+  std::vector<int> start(DP_MAX_WINDOW + 2, 0);
+  if (distinct > 1) {  // clip ids grouped by phase, ascending within a phase (a counting sort)
+    for (int s = 0; s <= DP_MAX_WINDOW; ++s) start[s + 1] = start[s] + count[s];
+    std::vector<int> at(start.begin(), start.end() - 1);
+    for (int c = 0; c < B; ++c) h_class[at[phase[c]]++] = c;
+  }
+  CK(cudaMemcpyAsync(e->d_restart, h_ids, (size_t)n * 4, cudaMemcpyHostToDevice, st));
+  if (distinct > 1) CK(cudaMemcpyAsync(e->d_class, h_class, (size_t)B * 4, cudaMemcpyHostToDevice, st));
+  float* d_state = reinterpret_cast<float*>(e->d_restart + cap * 8);
+  CK(cudaMemcpyAsync(d_state, h_state, (size_t)n * DP_RESTART_STATE * 4, cudaMemcpyHostToDevice, st));
+  CK(cudaEventRecord(e->ev_restart, st));
+  e->restart_pending = true;
+  const int32_t* d_ids = reinterpret_cast<const int32_t*>(e->d_restart);
+  CK(dp_reset_clips_launch(d_ids, d_state, n, e->d_latent, e->d_gpos, e->d_grot, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, st));
+  ++e->launches;
+  if (W == 0 && e->target_rows == 1 && e->look_left > 0) {
+    // Window 0 between look-ahead boundaries: the restarted clips need targets for the rest of the current four-frame cycle.  What
+    // the predictor reads at their own frames 0..3 (chronological ring rows <= 56) is all initial rows, so one single-view call on
+    // them, broadcast into rows look_next..3, is what the reference computes frame by frame.
+    const int rc = predict_subset(e, d_ids, n, 0, e->d_target_pre, DP_LOOKAHEAD, e->look_next, 0, st);
+    if (rc) return rc;
+  }
+  if (distinct == 1) {  // one phase for every clip: fold it into current_index (lockstep path, prefetch and graph replay stay on)
+    std::fill(e->phase.begin(), e->phase.end(), 0);
+    e->current_index = 0;  // that phase is g: every clip starts its own window at the next frame
+  } else {
+    std::copy(phase.begin(), phase.end(), e->phase.begin());
+    e->class_start = start;
+  }
+  e->n_phases = distinct;
+  return DP_OK;
+}
+
+extern "C" int dp_engine_get_clip_index(dp_engine* e, int window, int32_t* index) {
+  if (!e || !index) return fail(DP_ERR_ARG, "dp_engine_get_clip_index: null argument");
+  if (window < 0 || window > DP_MAX_WINDOW || window % 4) return fail(DP_ERR_ARG, "window must be a multiple of 4 in [0,116]");
+  if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
+  const bool same = e->target_rows == window + 1;
+  if (!same && e->n_phases > 1) return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own phase");
+  // a window change keeps the index unless it lies beyond the new buffer (run_one)
+  const int g = window == 0 ? 0 : (!same && e->current_index > window ? 0 : e->current_index);
+  for (int c = 0; c < e->n_clips; ++c) index[c] = window == 0 ? 0 : (g - e->phase[c] + window) % window;
+  return DP_OK;
+}
+
+extern "C" int dp_engine_frames_to_boundary(const dp_engine* e, int window) {
+  if (!e) return fail(DP_ERR_ARG, "null engine");
+  if (window < 0 || window > DP_MAX_WINDOW || window % 4) return fail(DP_ERR_ARG, "window must be a multiple of 4 in [0,116]");
+  if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
+  const bool same = e->target_rows == window + 1;
+  if (!same && e->n_phases > 1) return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own phase");
+  if (window == 0) return same ? e->look_left : 0;  // the next look-ahead call covers every clip
+  // the next frame whose index is some clip's phase: a predictor call runs there anyway, a clip restarted just before joins it
+  int g = !same && e->current_index > window ? 0 : e->current_index;
+  for (int d = 0; d <= window; ++d, g = (g + 1) % window)
+    if (e->n_phases > 1 ? e->class_start[g + 1] > e->class_start[g] : g == 0) return d;
+  return fail(DP_ERR_STATE, "dp_engine_frames_to_boundary: no predictor frame ahead");
+}

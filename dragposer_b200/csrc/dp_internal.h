@@ -78,3 +78,14 @@ cudaError_t dp_ff_tc_launch(const unsigned char* wimg, const float* blob, const 
 cudaError_t dp_encode_launch(const float* blob, const float* dqs, const float* eps, float* latent, int n, cudaStream_t st);
 // per row: mean joint distance, mean end-effector distance of two poses in the engine's output format (root at the origin)
 cudaError_t dp_pose_error_launch(const DpModelImage* model, const float* pose_a, const float* pose_b, int n, float* err, cudaStream_t st);
+// Per-clip restarts (dp_restart.cu).  state: n rows of latent (24) | global_pos (3) | global_rot (4) | heights (6)
+#define DP_RESTART_STATE (DP_L + 3 + 4 + DP_NH)
+cudaError_t dp_reset_clips_launch(const int32_t* ids, const float* state, int n, float* latent, float* gpos, float* grot,
+                                  float* latent_buf, float* disp_buf, float* height_buf, cudaStream_t st);
+// ring rows of the listed clips -> compact (n, DP_PAST, .) buffers, slot for slot
+cudaError_t dp_gather_rings_launch(const int32_t* ids, int n, const float* latent_buf, const float* disp_buf, const float* height_buf,
+                                   float* s_latent, float* s_disp, float* s_height, cudaStream_t st);
+// compact predictor rows (n, src_rows, 24) -> rows [r0, dst_rows) of the listed clips' target rows; src_rows == 1 broadcasts,
+// otherwise own row k < window goes to slot (k + shift) % window and own row `window` to slot `window`
+cudaError_t dp_scatter_targets_launch(const float* src, int src_rows, const int32_t* ids, int n, float* dst, int dst_rows, int r0,
+                                      int window, int shift, cudaStream_t st);

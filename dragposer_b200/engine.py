@@ -176,6 +176,34 @@ class BatchedDragPose:
         initialise the clips (ring buffers tiled with the initial latent / heights)."""
         self.set_initial_state(self.encode(dqs, eps), global_pos, global_rot, heights)
 
+    def restart_clips(self, clips, latent, global_pos, global_rot, heights):
+        """Restart the clips `clips` (unique ids < n_clips) with latent (n,24), global_pos (n,3), global_rot (n,4), heights (n,6),
+        like set_initial_state does for every clip, while the others keep running.  Each restarted clip's next frame is its own
+        frame 0.  Restarting when frames_to_boundary(window) == 0 keeps the lockstep path; elsewhere the restarted clips get
+        their own predictor phase (include/dp_engine.h:dp_engine_restart_clips)."""
+        ids = _i32(clips).reshape(-1)
+        n = ids.shape[0]
+        z, gp = _f32(latent).reshape(n, 24), _f32(global_pos).reshape(n, 3)
+        gr, ht = _f32(global_rot).reshape(n, 4), _f32(heights).reshape(n, 6)
+        _lib.check(self.lib.dp_engine_restart_clips(self.h, n, _ptr(ids), _ptr(z), _ptr(gp), _ptr(gr), _ptr(ht), None))
+
+    def restart_pose(self, clips, dqs, global_pos, global_rot, heights, eps=None):
+        """restart_clips with the latent encoded on the device from standardised dual quats (n,176) (see set_initial_pose)."""
+        self.restart_clips(clips, self.encode(dqs, eps), global_pos, global_rot, heights)
+
+    def clip_index(self, window):
+        """Own temporal index of every clip for the next frame run with `window` (B,) -- DragPose.current_index per clip."""
+        out = np.empty(self.n_clips, np.int32)
+        _lib.check(self.lib.dp_engine_get_clip_index(self.h, int(window), _ptr(out)))
+        return out
+
+    def frames_to_boundary(self, window):
+        """Frames until the next frame at which a restart costs no extra predictor call (0 = the next frame)."""
+        rc = self.lib.dp_engine_frames_to_boundary(self.h, int(window))
+        if rc < 0:
+            _lib.check(rc)
+        return int(rc)
+
     def pose_error(self, pose_a, pose_b):
         """Per-row MPJPE and MPEEPE (metres) between two sets of poses in the engine's output format (n,88), computed on the
         device (eval_metrics.py:6-32 with the root at the origin) -> (mpjpe (n,), mpeepe (n,))."""

@@ -1,6 +1,7 @@
 """Drop-in for the reference's evaluation CLI (python/src/eval_drag.py:255-293):
 
     python -m dragposer_b200.eval_drag <model_dir | folded.npz> <file.bvh | dir> [--config cfg.json] [--verbose]
+                                       [--batch [--slots N]]
 
 Same arguments, same JSON tracker-config keys, same printed metrics; writes `data/eval_<name>.bvh`.  The per-frame
 optimisation runs on the B200 engine; target construction from the ground-truth clip and the BVH/metric export are
@@ -131,6 +132,125 @@ def evaluate_batch(model_path, input_paths, config=None, save=False, seed=2222, 
     return results
 
 
+LOOKAHEAD = 4  # frames of one look-ahead predictor cycle at window 0 (DP_LOOKAHEAD, csrc/dp_internal.h)
+
+
+def boundary_period(window):
+    """Frames between two frames at which a clip can start without an extra predictor call: the window, or the look-ahead cycle
+    at window 0."""
+    return window if window > 0 else LOOKAHEAD
+
+
+def slot_schedule(lengths, slots, period):
+    """Continuous batching of clips of `lengths` frames over `slots` engine rows.  The first `slots` clips start at frame 0; every
+    later clip, in order, takes the slot that frees first (lowest slot on a tie) at the first multiple of `period` at or after that
+    slot's clip has ended, so a slot idles at most period - 1 frames.  Returns (starts, total): starts[i] = (slot, first engine
+    frame) of clip i, which runs engine frames [first, first + lengths[i]); total = engine frames of the whole run."""
+    import heapq
+
+    free = [(0, s) for s in range(min(slots, len(lengths)))]
+    starts = []
+    for n in lengths:
+        t, s = heapq.heappop(free)
+        t = -(-t // period) * period
+        starts.append((s, t))
+        heapq.heappush(free, (t + int(n), s))
+    return starts, max((t + int(n) for (_, t), n in zip(starts, lengths)), default=0)
+
+
+def evaluate_stream(model_path, input_paths, slots, config=None, save=False, seed=2222, initial_latents=None, max_frames=None, device=0,
+                    random_temporal=False, predictor_path=0):
+    """Many BVH clips through a fixed number of engine rows (continuous batching): a slot whose clip has ended takes the next file
+    at the next predictor boundary (slot_schedule), with BatchedDragPose.restart_pose / restart_clips, so the batch stays on the
+    lockstep path and no frame is padded beyond the wait for that boundary.  Targets are world-space (targets_world=True) and are
+    built per run of frames between two restarts.  Same optimiser settings, metrics and result dicts as evaluate_batch(); frames a
+    slot spends waiting are computed and discarded.  predictor_path: 0 = tensor-core predictor, 1 = fp32 CUDA-core kernels."""
+    from .engine import BatchedDragPose
+
+    torch.manual_seed(seed)
+    np.random.seed(seed)
+    cfg = synthetic.TrackerConfig.load(config) if config else synthetic.config_6_trackers()
+    bvhs = [Bvh(p) for p in input_paths]
+    parents, offsets = bvhs[0].skeleton()
+    for b in bvhs[1:]:
+        p2, o2 = b.skeleton()
+        if list(p2) != list(parents) or not np.allclose(o2, offsets, atol=1e-6):
+            raise ValueError("evaluate_stream: all clips must share one skeleton")
+    pm = dpm.load_pose_model(model_path, parents)
+    tdir = model_path if os.path.isdir(model_path) else os.path.dirname(model_path)
+    tm = dpm.load_temporal_model(tdir, allow_random=random_temporal)
+    joints, weights = cfg.joints, cfg.tracker_weights
+    rots = [b.quaternions() for b in bvhs]
+    clips = [motion.ClipData(r, b.positions[:, 0, :], parents, offsets, pm.mean_dqs, pm.std_dqs) for r, b in zip(rots, bvhs)]
+    lens = [c.n_frames if max_frames is None else min(max_frames, c.n_frames) for c in clips]
+    W = cfg.temporal_future_window
+    starts, total = slot_schedule(lens, slots, boundary_period(W))
+    N, E = min(slots, len(clips)), len(joints)
+    eng = BatchedDragPose(pm, offsets, tm, N, device=device)
+    eng.set_predictor_path(predictor_path)
+    if initial_latents is not None:
+        latent0 = [np.asarray(z, np.float32).reshape(24) for z in initial_latents]
+        eps = None
+    else:  # one torch draw per clip in clip order, like evaluate_batch; encoded on the device when the clip starts
+        eps = [torch.randn(1, dpm.LATENT).numpy() for _ in clips]
+
+    def begin(ids, first):  # clips `ids` start now in their slots
+        rows = [starts[i][0] for i in ids]
+        state = (np.stack([clips[i].global_pos[0] for i in ids]), np.stack([clips[i].global_rot[0] for i in ids]),
+                 np.stack([clips[i].heights[0] for i in ids]))
+        if eps is None:
+            z = np.stack([latent0[i] for i in ids])
+        else:
+            z = eng.encode(np.stack([clips[i].dqs[0] for i in ids]), np.concatenate([eps[i] for i in ids]))
+        if first:
+            eng.set_initial_state(z, *state)
+        else:
+            assert eng.frames_to_boundary(W) == 0
+            eng.restart_clips(rows, z, *state)
+
+    opts = dict(stop_eps_pos=0.01 * 0.01, stop_eps_rot=0.01, max_iter=100, min_loss_incr=0.00001, learning_rate=1e-2, lambda_rot=1,
+                lambda_temporal=cfg.lambda_temporal, temporal_future_window=W, joint_adjustment_indices=cfg.joint_adjustment,
+                joint_adjustment_weight=cfg.joint_adjustment_weight, targets_world=True)
+    poses = [np.empty((n, 88), np.float32) for n in lens]
+    gposs = [np.empty((n, 3), np.float32) for n in lens]
+    by_start = {}
+    for i, (_, t) in enumerate(starts):
+        by_start.setdefault(t, []).append(i)
+    cuts = sorted(by_start) + [total]
+    current = [None] * N  # clip in each slot
+    targets = {}  # world-space targets of the clips running now
+    elapsed = 0.0
+    for a, b in zip(cuts[:-1], cuts[1:]):
+        for i in by_start[a]:
+            targets.pop(current[starts[i][0]], None)  # the slot's previous clip, kept until now for the frames spent waiting
+            current[starts[i][0]] = i
+            targets[i] = motion.world_targets(clips[i], pm.mean_q, pm.std_q, parents, offsets, joints, lens[i])
+        begin(by_start[a], a == 0)
+        tp, tr = np.empty((b - a, N, E, 3), np.float32), np.empty((b - a, N, E, 3, 3), np.float32)
+        for s, i in enumerate(current):
+            f = np.minimum(np.arange(a, b) - starts[i][1], lens[i] - 1)  # a slot waiting for the boundary repeats its last frame
+            tp[:, s], tr[:, s] = targets[i][0][f], targets[i][1][f]
+        t0 = time.time()
+        p, g = eng.run_frames(tp, tr, joints, weights, **opts)
+        elapsed += time.time() - t0
+        for s, i in enumerate(current):
+            f0, f1 = a - starts[i][1], min(b - starts[i][1], lens[i])
+            if f1 > f0:
+                poses[i][f0:f1], gposs[i][f0:f1] = p[: f1 - f0, s], g[: f1 - f0, s]
+    eng.close()
+    results = []
+    for i, (bvh, c) in enumerate(zip(bvhs, clips)):
+        local = motion.result_local_quats(poses[i], pm.mean_q, pm.std_q, parents)
+        out_path = None
+        if save:
+            os.makedirs("data", exist_ok=True)
+            out_path = os.path.join("data", "eval_" + os.path.basename(input_paths[i]))
+            write_result_bvh(bvh, local, gposs[i], out_path)
+        m, e = motion.mpjpe(rots[i][: lens[i]], local.astype(np.float64), np.asarray(offsets, np.float64), parents)
+        results.append(dict(mpjpe=m, mpeepe=e, time=elapsed, poses=poses[i], global_pos=gposs[i], out_path=out_path))
+    return results
+
+
 def write_result_bvh(bvh: Bvh, local_quats, root_pos, path):
     F = local_quats.shape[0]
     with open(path, "w") as fh:
@@ -179,13 +299,19 @@ def main():
     ap.add_argument("--verbose", action="store_true", default=False, help="print additional information")
     ap.add_argument("--batch", action="store_true", default=False,
                     help="directory input: run all clips together as one batch (one engine row per clip, world-space targets)")
+    ap.add_argument("--slots", type=int, default=0,
+                    help="with --batch: run the clips through this many engine rows, a new clip starting in a slot whose clip has ended")
     ap.add_argument("--random-temporal", action="store_true", default=False,
                     help="temporal.pt is missing: run with the seed-2222 random-init predictor instead of failing like the reference")
     args = ap.parse_args()
     rt = args.random_temporal
     if os.path.isdir(args.input_path) and args.batch:
         files = [os.path.join(args.input_path, fn) for fn in sorted(os.listdir(args.input_path)) if fn.endswith(".bvh")]
-        for fn, r in zip(files, evaluate_batch(args.model_path, files, args.config, save=True, quiet=True, random_temporal=rt)):
+        if args.slots > 0:
+            results = evaluate_stream(args.model_path, files, args.slots, args.config, save=True, random_temporal=rt)
+        else:
+            results = evaluate_batch(args.model_path, files, args.config, save=True, quiet=True, random_temporal=rt)
+        for fn, r in zip(files, results):
             print("Evaluate {} ------------------------".format(fn))
             print("Evaluate Loss: {}".format(r["mpjpe"] + r["mpeepe"]))
             print("Mean Per Joint Position Error: {}".format(r["mpjpe"]))

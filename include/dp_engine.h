@@ -229,6 +229,22 @@ int dp_engine_encode_host(dp_engine* e, int n, const float* dqs, const float* ep
  * skeletons with the root at the origin.  HOST pointers. */
 int dp_engine_pose_error_host(dp_engine* e, int n, const float* pose_a, const float* pose_b, float* err);
 
+/* Per-clip restarts of a running batch.
+ * Restart n clips (ids unique, < n_clips) like DragPose.set_initial_pose, leaving every other clip untouched; each restarted clip's
+ * next frame is its own frame 0 (predictor call, look-ahead, ring).  latent0 (n,24), global_pos (n,3), global_rot (n,4 wxyz),
+ * heights (n,6).  HOST pointers; enqueued on `stream` (NULL = engine stream), which must be the stream the frames run on.
+ * A restart at a boundary (dp_engine_frames_to_boundary == 0) keeps every clip at one predictor phase and adds one kernel.
+ * Anywhere else the restarted clips run at their own phase: their predictor calls then run separately, on the frame's stream
+ * (no early call in the small-batch mode), and until every clip shares one phase again (dp_engine_init_clips, or restarts) a
+ * window change or dp_engine_predict_targets fails with DP_ERR_STATE.  dp_engine_get_state keeps reporting the global
+ * current_index and returns target_buf in each clip's own row order. */
+int dp_engine_restart_clips(dp_engine* e, int n, const int32_t* clips, const float* latent0, const float* global_pos,
+                            const float* global_rot, const float* heights, void* stream);
+/* Own temporal index of every clip for the next frame run with `window` (B) -- what DragPose.current_index would be. */
+int dp_engine_get_clip_index(dp_engine* e, int window, int32_t* index);
+/* Frames until the next frame at which a restart costs no extra predictor call (0 = the next frame), or a negative dp_status. */
+int dp_engine_frames_to_boundary(const dp_engine* e, int window);
+
 /* Number of kernels launched by this engine since creation (bench "gpu_launches"). */
 long long dp_engine_launch_count(const dp_engine* e);
 
