@@ -282,14 +282,15 @@ def temporal_forward(sd, enc_in, dec_in, n_enc=3, n_dec=3):
 
 
 def predict_targets(sd, means_latent, stds_latent, latent_buf, disp_buf, height_buf, window):
-    """Ring buffers (B,60,·) in chronological order -> target_latent_buffer (B,W+1,24)."""
+    """Ring buffers (B,60,·) in chronological order -> target_latent_buffer (B,W+1,24), in the dtype of the ring buffers
+    (float64 rings, statistics and state dict give a float64 predictor)."""
     idx = PAST_INDEX
     lat = (latent_buf[:, idx[:-1]] - means_latent) / stds_latent
     dacc = torch.stack([disp_buf[:, j : j + SAMPLE_STEP].sum(1) for j in idx[:-1]], 1)
     enc_in = torch.cat((lat, dacc, height_buf[:, idx[:-1]]), -1)
     dec_in = ((latent_buf[:, idx[-1]] - means_latent) / stds_latent)[:, None]
     B = latent_buf.shape[0]
-    buf = torch.zeros(B, window + 1, 24)
+    buf = torch.zeros(B, window + 1, 24, dtype=latent_buf.dtype)
     with torch.no_grad():
         for i in range(0, window + 1, SAMPLE_STEP):
             out = temporal_forward(sd, enc_in, dec_in)
