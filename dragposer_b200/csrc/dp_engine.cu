@@ -19,7 +19,6 @@
 #include "../../include/dp_engine.h"
 #include "dp_internal.h"
 
-#define DP_AUTO_TC_PATH 3  // tensor-core variant picked by decoder_path = 0 for batches
 static thread_local std::string g_err;
 static int fail(int code, const std::string& msg) {
   g_err = msg;
@@ -30,6 +29,49 @@ static int fail(int code, const std::string& msg) {
     cudaError_t _e = (call);                                                                       \
     if (_e != cudaSuccess) return fail(DP_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_e)); \
   } while (0)
+
+static int check_window(int w) {  // drag_pose.py:236
+  return (w < 0 || w > DP_MAX_WINDOW || w % 4) ? fail(DP_ERR_ARG, "the temporal window must be a multiple of 4 in [0,116]") : DP_OK;
+}
+
+// Which target row every clip reads at the next frame and when the predictor runs (drag_pose.py:237-244,399-402); host state only.
+// Look-ahead at temporal_future_window == 0 (the predictor runs every frame): its inputs end three frames in the past
+// (train_temporal.param["past_frames"] stops at ring row 56 of 60), so the targets of this frame AND the next three are computed
+// in ONE batched predictor call (4 x n_clips virtual clips: fuller tiles, a quarter of the launches) -- the same numbers the
+// reference computes frame by frame.
+// Per-clip restarts (dp_engine_restart_clips).  Clip c runs at its own predictor phase phase[c]: its own temporal index is
+// (current_index - phase[c]) mod window, and its own target row k < window lives in slot (k + phase[c]) % window of d_target_buf
+// (row window in slot window), so the frame kernels read slot current_index of every clip as before.  While every clip shares one
+// phase it is folded into current_index (all phases 0, n_phases 1) and nothing differs from a batch that was never restarted.
+struct TargetSchedule {
+  int target_rows = 0;           // window + 1 of d_target_buf, 0 = none yet
+  int current_index = 0;
+  int look_left = 0;             // window 0: rows of d_target_pre not read yet; the next frame reads row DP_LOOKAHEAD - look_left
+  int look_last_row = -1;        // window 0: the row of d_target_pre the last frame read; -1 = it read d_target_buf
+  std::vector<int> phase;        // (n_clips)
+  int n_phases = 1;              // distinct phases among the clips; >= 2 = mixed
+  std::vector<int> class_start;  // mixed phases: the clips of phase s are d_class[class_start[s] .. class_start[s + 1])
+  // The index a frame at window W runs at.  The reference keeps current_index when the window changes: rows of the fresh zero buffer
+  // are used until it wraps to 0.  An index beyond the new buffer, an IndexError there on every later frame, restarts the cycle here.
+  int index_at(int W) const { return current_index > W ? 0 : current_index; }
+  int check_window_change(int W) const {
+    if (target_rows != W + 1 && n_phases > 1)
+      return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own predictor phase: "
+                                "re-initialise the clips (dp_engine_init_clips) to change it");
+    return DP_OK;
+  }
+  int clip_index(int c, int W) const { return W == 0 ? 0 : (index_at(W) - phase[c] + W) % W; }
+  int slot(int c, int k, int W) const { return (k + phase[c]) % W; }  // of clip c's own row k < W
+  // The next frame whose index is some clip's phase: a predictor call runs there anyway, a clip restarted just before joins it.
+  int frames_to_boundary(int W) const {
+    if (W == 0) return target_rows == 1 ? look_left : 0;  // the next look-ahead call covers every clip
+    for (int d = 0, g = index_at(W); d <= W; ++d, g = (g + 1) % W)
+      if (n_phases > 1 ? class_start[g + 1] > class_start[g] : g == 0) return d;
+    return fail(DP_ERR_STATE, "dp_engine_frames_to_boundary: no predictor frame ahead");
+  }
+  void reset(int n_clips) { *this = TargetSchedule(); phase.assign(n_clips, 0); }
+  void advance(int W) { current_index = W == 0 ? 0 : (current_index + 1) % W; }  // drag_pose.py:399-402
+};
 
 struct dp_engine {
   int device = 0, max_clips = 0, n_clips = 0, num_sms = 148;
@@ -48,15 +90,9 @@ struct dp_engine {
   float *d_latent = nullptr, *d_gpos = nullptr, *d_grot = nullptr;
   float *d_latent_buf = nullptr, *d_disp_buf = nullptr, *d_height_buf = nullptr;
   float* d_target_buf = nullptr;  // (B, DP_MAX_WINDOW+1, 24) capacity; logical rows = window+1
-  int target_rows = 0;            // window + 1 of the current buffer, 0 = none yet
   int ring_head = 0;
-  int current_index = 0;
-  // Look-ahead at temporal_future_window == 0 (the predictor runs every frame): its inputs end three frames in the past
-  // (train_temporal.param["past_frames"] stops at ring row 56 of 60), so the targets of this frame AND the next three are computed
-  // in ONE batched predictor call (4 x n_clips virtual clips: fuller tiles, a quarter of the launches) -- the same numbers the
-  // reference computes frame by frame.
-  float* d_target_pre = nullptr;  // (B, DP_LOOKAHEAD, 24)
-  int look_left = 0, look_next = 0, look_last_row = -1;
+  float* d_target_pre = nullptr;  // (B, DP_LOOKAHEAD, 24): the window-0 look-ahead rows (TargetSchedule)
+  TargetSchedule sched;
   // Predictor ahead of time in the small-batch streaming mode (window >= 4, <= DP_PREFETCH_MAX_CLIPS clips; DP_PRED_PREFETCH=0 turns it
   // off).  The same three-frame slack as above: what the predictor reads at the window's first frame t (chronological ring rows
   // 0..56) is complete once frame t-4 is, so the call for frame t is issued three frames early, on its own stream, with the ring head
@@ -66,8 +102,8 @@ struct dp_engine {
   float* d_target_alt = nullptr;
   cudaStream_t pre_stream = nullptr;
   cudaEvent_t ev_pre_fork = nullptr, ev_pre_done = nullptr;
-  bool pre_valid = false;
-  int pre_window = -1, prefetch = 1;
+  bool pre_valid = false;  // an early call into d_target_alt was issued at the current window and not used yet
+  int prefetch = 1;
   // outputs / diagnostics
   int32_t* d_iters = nullptr;
   float* d_losses = nullptr;
@@ -92,14 +128,7 @@ struct dp_engine {
   int profiling = 0;
   unsigned long long* d_phase = nullptr;  // 8 phase-cycle counters + 48 timeline stamps of the tcgen05 frame kernel (profiling level 2 only)
   std::vector<cudaEvent_t> prof_events;  // triples: before predictor, before frame kernel, after frame kernel
-  // Per-clip restarts (dp_engine_restart_clips).  Clip c runs at its own predictor phase phase[c]: its own temporal index is
-  // (current_index - phase[c]) mod window, and its own target row k < window lives in slot (k + phase[c]) % window of d_target_buf
-  // (row window in slot window), so the frame kernels read slot current_index of every clip as before.  While every clip shares one
-  // phase it is folded into current_index (all phases 0, n_phases 1) and nothing differs from a batch that was never restarted.
-  std::vector<int> phase;        // (max_clips)
-  int n_phases = 1;              // distinct phases among the clips; >= 2 = mixed
-  std::vector<int> class_start;  // mixed phases: the clips of phase s are d_class[class_start[s] .. class_start[s + 1])
-  int32_t* d_class = nullptr;    // clip ids grouped by phase, ascending within a phase
+  int32_t* d_class = nullptr;  // restarts: clip ids grouped by phase (TargetSchedule::class_start), ascending within a phase
   // pinned staging of a restart: restarted ids (max_clips) | ids grouped by phase (max_clips) | state rows (max_clips, DP_RESTART_STATE);
   // ev_restart follows its copies, so the next restart does not overwrite a block still in flight
   unsigned char *h_restart = nullptr, *d_restart = nullptr;
@@ -111,11 +140,15 @@ struct dp_engine {
 
 extern "C" const char* dp_engine_last_error(void) { return g_err.c_str(); }
 #define DP_PREFETCH_MAX_CLIPS 256
-// targets computed ahead of time are void (ring rows, model, path, window or clip set changed), or the predictor's work buffers are
-// about to be used by someone else: let the early call finish and forget it
+// let the early call finish and forget it: its targets are void (window or clips changed) or its work buffers are needed elsewhere
 static void drop_prefetch(dp_engine* e) {
   if (e->pre_valid) cudaStreamSynchronize(e->pre_stream);
   e->pre_valid = false;
+}
+
+static void void_targets_ahead(dp_engine* e) {  // the early call and the look-ahead rows: ring rows, clips, model or path changed
+  drop_prefetch(e);
+  e->sched.look_left = 0;
 }
 
 extern "C" int dp_engine_version(void) { return 100; }
@@ -173,8 +206,6 @@ extern "C" int dp_engine_create(dp_engine** out, int device, int max_clips) {
   CK(cudaEventCreateWithFlags(&e->tw.ev_fork, cudaEventDisableTiming));
   CK(cudaStreamCreateWithFlags(&e->tw.st_extra, cudaStreamNonBlocking));
   CK(cudaEventCreateWithFlags(&e->tw.ev_join, cudaEventDisableTiming));
-  e->phase.assign(B, 0);
-  e->class_start.assign(DP_MAX_WINDOW + 2, 0);
   *out = e;
   return DP_OK;
 }
@@ -352,7 +383,7 @@ extern "C" int dp_engine_set_temporal_model(dp_engine* e, const float* blob, siz
   if (!e || !blob || !means_latent || !stds_latent) return fail(DP_ERR_ARG, "dp_engine_set_temporal_model: null argument");
   if (n_floats != e->tl.total) return fail(DP_ERR_ARG, "dp_engine_set_temporal_model: blob size mismatch");
   CK(cudaSetDevice(e->device));
-  drop_prefetch(e);
+  void_targets_ahead(e);
   if (!e->d_tblob) CK(cudaMalloc(&e->d_tblob, n_floats * 4));
   CK(cudaMemcpy(e->d_tblob, blob, n_floats * 4, cudaMemcpyHostToDevice));
   CK(cudaMemcpy(e->d_mu, means_latent, DP_L * 4, cudaMemcpyHostToDevice));
@@ -374,7 +405,6 @@ extern "C" int dp_engine_set_temporal_model(dp_engine* e, const float* blob, siz
     if (!e->d_fftiles) CK(cudaMalloc(&e->d_fftiles, tiles.size()));
     CK(cudaMemcpy(e->d_fftiles, tiles.data(), tiles.size(), cudaMemcpyHostToDevice));
   }
-  e->look_left = 0;
   e->has_temporal = true;
   dp_temporal_graphs_clear(e->tw.graphs);
   return DP_OK;
@@ -386,7 +416,7 @@ extern "C" int dp_engine_init_clips(dp_engine* e, int n, const float* latent0, c
   if (n <= 0 || n > e->max_clips) return fail(DP_ERR_ARG, "dp_engine_init_clips: n_clips out of range");
   CK(cudaSetDevice(e->device));
   CK(cudaStreamSynchronize(e->stream));
-  drop_prefetch(e);
+  void_targets_ahead(e);
   std::vector<float> lb((size_t)n * DP_PAST * DP_L), hb((size_t)n * DP_PAST * DP_NH);
   for (int c = 0; c < n; ++c)
     for (int r = 0; r < DP_PAST; ++r) {
@@ -401,12 +431,7 @@ extern "C" int dp_engine_init_clips(dp_engine* e, int n, const float* latent0, c
   CK(cudaMemset(e->d_disp_buf, 0, (size_t)n * DP_PAST * 3 * 4));
   e->n_clips = n;
   e->ring_head = 0;
-  e->current_index = 0;
-  e->target_rows = 0;
-  e->look_left = 0;
-  e->look_last_row = -1;
-  std::fill(e->phase.begin(), e->phase.end(), 0);
-  e->n_phases = 1;
+  e->sched.reset(n);
   return DP_OK;
 }
 
@@ -446,8 +471,7 @@ static int check_params(const dp_engine* e, const dp_run_params* p, int ee_strid
   if (!e->has_pose) return fail(DP_ERR_STATE, "pose model not set");
   if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
   if (p->max_iter < 1 || p->max_iter > DP_MAX_ITER) return fail(DP_ERR_ARG, "max_iter out of range");
-  if (p->temporal_future_window < 0 || p->temporal_future_window > DP_MAX_WINDOW || p->temporal_future_window % 4)
-    return fail(DP_ERR_ARG, "temporal_future_window must be a multiple of 4 in [0,116]");  // drag_pose.py:236
+  if (int rc = check_window(p->temporal_future_window)) return rc;
   if (ee_stride < 1 || ee_stride > DP_JOINTS) return fail(DP_ERR_ARG, "ee_stride out of range");
   if (p->joint_adjust_joint >= DP_JOINTS || (p->joint_adjust_joint >= 0 && (p->joint_adjust_slot < 0 || p->joint_adjust_slot >= ee_stride)))
     return fail(DP_ERR_ARG, "joint adjustment indices out of range");
@@ -469,30 +493,44 @@ static int check_n_ee(const int32_t* n_ee, size_t count, int ee_stride, const dp
   return DP_OK;
 }
 
-static int ensure_subset_scratch(dp_engine* e) {
-  if (e->d_sub_target) return DP_OK;
-  const size_t B = (size_t)e->max_clips;
-  CK(cudaMalloc(&e->d_sub_latent, B * DP_PAST * DP_L * 4));
-  CK(cudaMalloc(&e->d_sub_disp, B * DP_PAST * 3 * 4));
-  CK(cudaMalloc(&e->d_sub_height, B * DP_PAST * DP_NH * 4));
-  CK(cudaMalloc(&e->d_sub_target, B * (DP_MAX_WINDOW + 1) * DP_L * 4));
+// The one caller of the temporal predictor: n clips' rings read from `head` -> (n, J or window + 1, 24) targets at dst, on st.
+static int run_predictor(dp_engine* e, const float* latent, const float* disp, const float* height, int head, int n, int window,
+                         float* dst, cudaStream_t st, int J = 1) {
+  if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
+  drop_prefetch(e);  // an early call still in flight uses the same work buffers
+  CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, latent, disp, height, head, n, window, dst, e->tw,
+                     e->predictor_path == 1 ? nullptr : e->d_fftiles, st, &e->launches, J));
   return DP_OK;
 }
 
 // The predictor for the n clips listed at d_ids (device) alone: their ring rows are gathered into compact buffers (same ring head),
 // the unmodified predictor runs on those, and its (n, window + 1, 24) rows are scattered into rows [r0, dst_rows) of dst -- rotated
-// by `shift` (see dp_engine::phase), or broadcast when window is 0.
+// by `shift` (see TargetSchedule::phase), or broadcast when window is 0.
 static int predict_subset(dp_engine* e, const int32_t* d_ids, int n, int window, float* dst, int dst_rows, int r0, int shift,
                           cudaStream_t st) {
-  int rc = ensure_subset_scratch(e);
-  if (rc) return rc;
-  drop_prefetch(e);  // the predictor's work buffers
+  if (!e->d_sub_target) {
+    const size_t B = (size_t)e->max_clips;
+    CK(cudaMalloc(&e->d_sub_latent, B * DP_PAST * DP_L * 4));
+    CK(cudaMalloc(&e->d_sub_disp, B * DP_PAST * 3 * 4));
+    CK(cudaMalloc(&e->d_sub_height, B * DP_PAST * DP_NH * 4));
+    CK(cudaMalloc(&e->d_sub_target, B * (DP_MAX_WINDOW + 1) * DP_L * 4));
+  }
   CK(dp_gather_rings_launch(d_ids, n, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, e->d_sub_latent, e->d_sub_disp, e->d_sub_height, st));
   ++e->launches;
-  CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_sub_latent, e->d_sub_disp, e->d_sub_height, e->ring_head, n, window,
-                     e->d_sub_target, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles, st, &e->launches));
+  if (int rc = run_predictor(e, e->d_sub_latent, e->d_sub_disp, e->d_sub_height, e->ring_head, n, window, e->d_sub_target, st)) return rc;
   CK(dp_scatter_targets_launch(e->d_sub_target, window + 1, d_ids, n, dst, dst_rows, r0, window, shift, st));
   ++e->launches;
+  return DP_OK;
+}
+
+// drag_pose.py:237-244: a fresh zero buffer when the window changes, at the index TargetSchedule::index_at gives
+static int set_window(dp_engine* e, int W, cudaStream_t st) {
+  if (e->sched.target_rows == W + 1) return DP_OK;
+  if (int rc = e->sched.check_window_change(W)) return rc;
+  drop_prefetch(e);
+  CK(cudaMemsetAsync(e->d_target_buf, 0, (size_t)e->n_clips * (W + 1) * DP_L * 4, st));
+  e->sched.current_index = e->sched.index_at(W);
+  e->sched.target_rows = W + 1;
   return DP_OK;
 }
 
@@ -500,69 +538,52 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
                    int shared, const float* tgt_pos, const float* tgt_rot, int ee_stride, float* out_pose, float* out_gpos,
                    cudaStream_t st) {
   const int W = p->temporal_future_window;
-  if (e->target_rows != W + 1) {  // drag_pose.py:237-244: fresh zero buffer when the window changes
-    if (e->n_phases > 1)
-      return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own predictor phase: "
-                                "re-initialise the clips (dp_engine_init_clips) to change it");
-    drop_prefetch(e);
-    CK(cudaMemsetAsync(e->d_target_buf, 0, (size_t)e->n_clips * (W + 1) * DP_L * 4, st));
-    e->target_rows = W + 1;
-    // The reference keeps current_index: rows of the zero buffer are used until the index wraps to 0.  An index beyond the new
-    // buffer is an IndexError there (and stays one on every later frame); here the cycle restarts and the predictor runs now.
-    if (e->current_index > W) e->current_index = 0;
-  }
+  int rc = set_window(e, W, st);
+  if (rc) return rc;
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   if (e->profiling) {
     for (int i = 0; i < 3; ++i) CK(cudaEventCreate(&ev[i]));
     CK(cudaEventRecord(ev[0], st));
   }
-  const bool look = W == 0;
-  if (!look) {
-    e->look_left = 0;
-    e->look_last_row = -1;
-    if (e->n_phases > 1) {  // mixed phases: the clips whose own frame 0 this is get their targets, the others keep theirs
-      const int s = e->current_index, n = e->class_start[s + 1] - e->class_start[s];
-      if (n > 0) {
-        if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
-        const int rc = predict_subset(e, e->d_class + e->class_start[s], n, W, e->d_target_buf, W + 1, 0, s, st);
-        if (rc) return rc;
-      }
-    } else if (e->current_index == 0) {
-      if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
-      if (e->pre_valid && e->pre_window == W) {  // issued three frames ago into the other buffer
+  // the predictor call this frame needs first, if any, and the target rows it reads
+  TargetSchedule& s = e->sched;
+  const int g = s.current_index;
+  DpFrameArgs a{};
+  if (W == 0) {
+    if (s.look_left == 0) {  // targets of this frame and of the next DP_LOOKAHEAD - 1 frames in one call
+      rc = run_predictor(e, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, e->ring_head, e->n_clips, 0, e->d_target_pre, st, DP_LOOKAHEAD);
+      if (rc) return rc;
+      s.look_left = DP_LOOKAHEAD;
+    }
+    s.look_last_row = DP_LOOKAHEAD - s.look_left--;
+    a.target_buf = e->d_target_pre; a.target_rows = DP_LOOKAHEAD; a.target_index = s.look_last_row;
+  } else {
+    s.look_left = 0;
+    s.look_last_row = -1;
+    if (s.n_phases > 1) {  // mixed phases: the clips whose own frame 0 this is get their targets, the others keep theirs
+      const int n = s.class_start[g + 1] - s.class_start[g];
+      if (n > 0 && (rc = predict_subset(e, e->d_class + s.class_start[g], n, W, e->d_target_buf, W + 1, 0, g, st))) return rc;
+    } else if (g == 0) {
+      if (e->pre_valid) {  // issued three frames ago into the other buffer
         CK(cudaStreamWaitEvent(st, e->ev_pre_done, 0));
         std::swap(e->d_target_buf, e->d_target_alt);
         e->pre_valid = false;
       } else {
-        drop_prefetch(e);
-        CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_latent_buf, e->d_disp_buf, e->d_height_buf,
-                           e->ring_head, e->n_clips, W, e->d_target_buf, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles, st,
-                           &e->launches));
+        rc = run_predictor(e, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, e->ring_head, e->n_clips, W, e->d_target_buf, st);
+        if (rc) return rc;
       }
-    } else if (e->prefetch && W >= 4 && e->current_index == W - 3 && e->n_clips <= DP_PREFETCH_MAX_CLIPS && e->has_temporal && !e->pre_valid) {
+    } else if (e->prefetch && g == W - 3 && e->n_clips <= DP_PREFETCH_MAX_CLIPS && e->has_temporal && !e->pre_valid) {
       // three frames before the window's first frame: every ring row that frame's predictor call will read is final (frame t-4 is
       // the newest one in the ring, enqueued on st before this point), and it will see the head three slots further on
       CK(cudaEventRecord(e->ev_pre_fork, st));
       CK(cudaStreamWaitEvent(e->pre_stream, e->ev_pre_fork, 0));
-      CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_latent_buf, e->d_disp_buf, e->d_height_buf,
-                         (e->ring_head + 3) % DP_PAST, e->n_clips, W, e->d_target_alt, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles,
-                         e->pre_stream, &e->launches));
+      rc = run_predictor(e, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, (e->ring_head + 3) % DP_PAST, e->n_clips, W, e->d_target_alt,
+                         e->pre_stream);
+      if (rc) return rc;
       CK(cudaEventRecord(e->ev_pre_done, e->pre_stream));
       e->pre_valid = true;
-      e->pre_window = W;
     }
-  } else {
-    drop_prefetch(e);
-    if (e->look_left == 0) {  // targets of this frame and of the next DP_LOOKAHEAD - 1 frames in one call
-      if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
-      CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_latent_buf, e->d_disp_buf, e->d_height_buf,
-                         e->ring_head, e->n_clips, 0, e->d_target_pre, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles, st,
-                         &e->launches, DP_LOOKAHEAD));
-      e->look_left = DP_LOOKAHEAD;
-      e->look_next = 0;
-    }
-    e->look_last_row = e->look_next++;
-    --e->look_left;
+    a.target_buf = e->d_target_buf; a.target_rows = W + 1; a.target_index = g;
   }
   if (e->trace_enabled && (!e->d_trace || e->trace_iters < p->max_iter)) {
     cudaFree(e->d_trace);
@@ -571,7 +592,6 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
     e->trace_iters = p->max_iter;
   }
   if (e->trace_enabled) CK(cudaMemsetAsync(e->d_trace, 0, (size_t)e->max_clips * e->trace_iters * 52 * 4, st));
-  DpFrameArgs a{};
   a.model = e->d_model;
   a.model_tc = e->d_model_tc;
   a.model_tmem = e->d_model_tmem;
@@ -579,8 +599,6 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
   a.latent = e->d_latent; a.gpos = e->d_gpos; a.grot = e->d_grot;
   a.latent_buf = e->d_latent_buf; a.disp_buf = e->d_disp_buf; a.height_buf = e->d_height_buf;
   a.ring_head = e->ring_head;
-  a.target_buf = e->d_target_buf; a.target_rows = W + 1; a.target_index = e->current_index;
-  if (look) { a.target_buf = e->d_target_pre; a.target_rows = DP_LOOKAHEAD; a.target_index = e->look_last_row; }
   a.n_ee = n_ee; a.joints = joints; a.weights = weights; a.shared_trackers = shared;
   a.tgt_pos = tgt_pos; a.tgt_rot = tgt_rot; a.ee_stride = ee_stride;
   a.targets_world = p->targets_world ? 1 : 0;
@@ -600,7 +618,7 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
   // kernel is the low-latency path for small batches (B = 1 streaming)
   a.ext_mask = p->extension_losses;
   a.floor_level = p->floor_level;
-  const int path = p->extension_losses ? 1 : (p->decoder_path ? p->decoder_path : (e->n_clips >= 512 ? DP_AUTO_TC_PATH : 1));
+  const int path = p->extension_losses ? 1 : (p->decoder_path ? p->decoder_path : (e->n_clips >= 512 ? 3 : 1));
   if (path == 3) CK(dp_frame_tc16_launch(a, e->num_sms, st));
   else CK(dp_frame_simt_launch(a, e->num_sms, st));
   e->last_path = path;
@@ -610,7 +628,7 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
     for (int i = 0; i < 3; ++i) e->prof_events.push_back(ev[i]);
   }
   e->ring_head = (e->ring_head + 1) % DP_PAST;
-  e->current_index = (W == 0) ? 0 : (e->current_index + 1) % W;  // drag_pose.py:399-402
+  e->sched.advance(W);
   return DP_OK;
 }
 
@@ -961,24 +979,23 @@ extern "C" int dp_engine_get_state(dp_engine* e, float* latent, float* gpos, flo
   if (latent_buf && (rc = copy_ring(e, e->d_latent_buf, latent_buf, DP_L))) return rc;
   if (disp_buf && (rc = copy_ring(e, e->d_disp_buf, disp_buf, 3))) return rc;
   if (height_buf && (rc = copy_ring(e, e->d_height_buf, height_buf, DP_NH))) return rc;
+  const TargetSchedule& s = e->sched;
   if (target_buf) {
-    if (e->target_rows <= 0) return fail(DP_ERR_STATE, "no target buffer yet");
-    if (e->look_last_row >= 0)  // window 0 with look-ahead: the row the last frame used, as (B,1,24)
-      CK(cudaMemcpy2D(target_buf, DP_L * 4, e->d_target_pre + (size_t)e->look_last_row * DP_L, (size_t)DP_LOOKAHEAD * DP_L * 4, DP_L * 4, B,
+    if (s.target_rows <= 0) return fail(DP_ERR_STATE, "no target buffer yet");
+    if (s.look_last_row >= 0)  // window 0 with look-ahead: the row the last frame used, as (B,1,24)
+      CK(cudaMemcpy2D(target_buf, DP_L * 4, e->d_target_pre + (size_t)s.look_last_row * DP_L, (size_t)DP_LOOKAHEAD * DP_L * 4, DP_L * 4, B,
                       cudaMemcpyDeviceToHost));
     else
-      CK(cudaMemcpy(target_buf, e->d_target_buf, B * e->target_rows * DP_L * 4, cudaMemcpyDeviceToHost));
-    if (e->n_phases > 1 && e->look_last_row < 0) {  // rotated rows (dp_engine::phase) -> each clip's own row order
-      const int W = e->target_rows - 1;
-      std::vector<float> own((size_t)W * DP_L);
-      for (size_t c = 0; c < B; ++c) {
-        float* rows = target_buf + c * e->target_rows * DP_L;
-        for (int k = 0; k < W; ++k) memcpy(&own[(size_t)k * DP_L], rows + (size_t)((k + e->phase[c]) % W) * DP_L, DP_L * 4);
-        memcpy(rows, own.data(), own.size() * 4);
+      CK(cudaMemcpy(target_buf, e->d_target_buf, B * s.target_rows * DP_L * 4, cudaMemcpyDeviceToHost));
+    if (s.n_phases > 1 && s.look_last_row < 0) {  // rotated rows (TargetSchedule::phase) -> each clip's own row order
+      const int W = s.target_rows - 1;
+      for (size_t c = 0; c < B; ++c) {  // own row k moves from slot(c, k) to k: rows [0, W) rotate left by slot(c, 0)
+        float* rows = target_buf + c * s.target_rows * DP_L;
+        std::rotate(rows, rows + (size_t)s.slot((int)c, 0, W) * DP_L, rows + (size_t)W * DP_L);
       }
     }
   }
-  if (current_index) *current_index = e->current_index;
+  if (current_index) *current_index = s.current_index;
   return DP_OK;
 }
 
@@ -992,8 +1009,7 @@ extern "C" int dp_engine_set_ring_buffers(dp_engine* e, const float* latent_buf,
   CK(cudaMemcpy(e->d_disp_buf, disp_buf, B * DP_PAST * 3 * 4, cudaMemcpyHostToDevice));
   CK(cudaMemcpy(e->d_height_buf, height_buf, B * DP_PAST * DP_NH * 4, cudaMemcpyHostToDevice));
   e->ring_head = 0;  // rows were given in chronological order
-  e->look_left = 0;  // targets computed ahead from the old rows are void
-  drop_prefetch(e);
+  void_targets_ahead(e);
   return DP_OK;
 }
 
@@ -1001,21 +1017,14 @@ extern "C" int dp_engine_predict_targets(dp_engine* e, int window, void* stream)
   if (!e) return fail(DP_ERR_ARG, "null engine");
   if (!e->has_temporal) return fail(DP_ERR_STATE, "temporal model not set");
   if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
-  if (window < 0 || window > DP_MAX_WINDOW || window % 4) return fail(DP_ERR_ARG, "window must be a multiple of 4 in [0,116]");
-  if (e->n_phases > 1)
+  if (int rc = check_window(window)) return rc;
+  if (e->sched.n_phases > 1)
     return fail(DP_ERR_STATE, "dp_engine_predict_targets: restarted clips run at their own predictor phase (it predicts every clip at once)");
   CK(cudaSetDevice(e->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-  drop_prefetch(e);  // this call uses the predictor's work buffers
-  if (e->target_rows != window + 1) {
-    CK(cudaMemsetAsync(e->d_target_buf, 0, (size_t)e->n_clips * (window + 1) * DP_L * 4, st));
-    e->target_rows = window + 1;
-  }
-  e->look_last_row = -1;  // dp_engine_get_state reports what this call writes
-  CK(dp_temporal_run(e->d_tblob, e->tl, e->d_mu, e->d_sigma, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, e->ring_head,
-                     e->n_clips, window, e->d_target_buf, e->tw, e->predictor_path == 1 ? nullptr : e->d_fftiles, st,
-                     &e->launches));
-  return DP_OK;
+  if (int rc = set_window(e, window, st)) return rc;
+  e->sched.look_last_row = -1;  // dp_engine_get_state reports what this call writes
+  return run_predictor(e, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, e->ring_head, e->n_clips, window, e->d_target_buf, st);
 }
 
 extern "C" int dp_engine_set_profiling(dp_engine* e, int enable) {
@@ -1069,8 +1078,7 @@ extern "C" int dp_engine_get_profile(dp_engine* e, double* ms_predictor, double*
 extern "C" int dp_engine_set_predictor_path(dp_engine* e, int path) {
   if (!e || path < 0 || path > 1) return fail(DP_ERR_ARG, "predictor path must be 0 (tcgen05 fp16x2 attention + FF) or 1 (fp32 CUDA-core kernels)");
   e->predictor_path = path;
-  e->look_left = 0;
-  drop_prefetch(e);
+  void_targets_ahead(e);
   return DP_OK;
 }
 
@@ -1102,9 +1110,9 @@ extern "C" int dp_engine_restart_clips(dp_engine* e, int n, const int32_t* clips
   e->restart_pending = false;
   drop_prefetch(e);  // targets computed ahead from the restarted clips' old rows are void
   // Each restarted clip's next frame is its own frame 0, i.e. its phase is the index the next frame runs at.
-  const int W = e->target_rows > 1 ? e->target_rows - 1 : 0;
-  const int g = e->current_index;
-  std::vector<int> phase(e->phase.begin(), e->phase.begin() + B);
+  TargetSchedule& sc = e->sched;
+  const int g = sc.current_index;
+  std::vector<int> phase = sc.phase;
   for (int i = 0; i < n; ++i) phase[clips[i]] = g;
   std::vector<int> count(DP_MAX_WINDOW + 1, 0);
   int distinct = 0;
@@ -1135,46 +1143,37 @@ extern "C" int dp_engine_restart_clips(dp_engine* e, int n, const int32_t* clips
   const int32_t* d_ids = reinterpret_cast<const int32_t*>(e->d_restart);
   CK(dp_reset_clips_launch(d_ids, d_state, n, e->d_latent, e->d_gpos, e->d_grot, e->d_latent_buf, e->d_disp_buf, e->d_height_buf, st));
   ++e->launches;
-  if (W == 0 && e->target_rows == 1 && e->look_left > 0) {
+  if (sc.target_rows == 1 && sc.look_left > 0) {
     // Window 0 between look-ahead boundaries: the restarted clips need targets for the rest of the current four-frame cycle.  What
     // the predictor reads at their own frames 0..3 (chronological ring rows <= 56) is all initial rows, so one single-view call on
-    // them, broadcast into rows look_next..3, is what the reference computes frame by frame.
-    const int rc = predict_subset(e, d_ids, n, 0, e->d_target_pre, DP_LOOKAHEAD, e->look_next, 0, st);
+    // them, broadcast into the rows from DP_LOOKAHEAD - look_left to 3, is what the reference computes frame by frame.
+    const int rc = predict_subset(e, d_ids, n, 0, e->d_target_pre, DP_LOOKAHEAD, DP_LOOKAHEAD - sc.look_left, 0, st);
     if (rc) return rc;
   }
   if (distinct == 1) {  // one phase for every clip: fold it into current_index (lockstep path, prefetch and graph replay stay on)
-    std::fill(e->phase.begin(), e->phase.end(), 0);
-    e->current_index = 0;  // that phase is g: every clip starts its own window at the next frame
+    std::fill(sc.phase.begin(), sc.phase.end(), 0);
+    sc.current_index = 0;  // that phase is g: every clip starts its own window at the next frame
   } else {
-    std::copy(phase.begin(), phase.end(), e->phase.begin());
-    e->class_start = start;
+    sc.phase = phase;
+    sc.class_start = start;
   }
-  e->n_phases = distinct;
+  sc.n_phases = distinct;
   return DP_OK;
 }
 
 extern "C" int dp_engine_get_clip_index(dp_engine* e, int window, int32_t* index) {
   if (!e || !index) return fail(DP_ERR_ARG, "dp_engine_get_clip_index: null argument");
-  if (window < 0 || window > DP_MAX_WINDOW || window % 4) return fail(DP_ERR_ARG, "window must be a multiple of 4 in [0,116]");
+  if (int rc = check_window(window)) return rc;
   if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
-  const bool same = e->target_rows == window + 1;
-  if (!same && e->n_phases > 1) return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own phase");
-  // a window change keeps the index unless it lies beyond the new buffer (run_one)
-  const int g = window == 0 ? 0 : (!same && e->current_index > window ? 0 : e->current_index);
-  for (int c = 0; c < e->n_clips; ++c) index[c] = window == 0 ? 0 : (g - e->phase[c] + window) % window;
+  if (int rc = e->sched.check_window_change(window)) return rc;
+  for (int c = 0; c < e->n_clips; ++c) index[c] = e->sched.clip_index(c, window);
   return DP_OK;
 }
 
 extern "C" int dp_engine_frames_to_boundary(const dp_engine* e, int window) {
   if (!e) return fail(DP_ERR_ARG, "null engine");
-  if (window < 0 || window > DP_MAX_WINDOW || window % 4) return fail(DP_ERR_ARG, "window must be a multiple of 4 in [0,116]");
+  if (int rc = check_window(window)) return rc;
   if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
-  const bool same = e->target_rows == window + 1;
-  if (!same && e->n_phases > 1) return fail(DP_ERR_STATE, "the temporal window cannot change while restarted clips run at their own phase");
-  if (window == 0) return same ? e->look_left : 0;  // the next look-ahead call covers every clip
-  // the next frame whose index is some clip's phase: a predictor call runs there anyway, a clip restarted just before joins it
-  int g = !same && e->current_index > window ? 0 : e->current_index;
-  for (int d = 0; d <= window; ++d, g = (g + 1) % window)
-    if (e->n_phases > 1 ? e->class_start[g + 1] > e->class_start[g] : g == 0) return d;
-  return fail(DP_ERR_STATE, "dp_engine_frames_to_boundary: no predictor frame ahead");
+  if (int rc = e->sched.check_window_change(window)) return rc;
+  return e->sched.frames_to_boundary(window);
 }

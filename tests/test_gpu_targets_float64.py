@@ -138,14 +138,17 @@ class ReferenceBookkeeping:
         self.bar[clips] = BAR_FLOOR
         self.idx[clips] = 0
 
-    def before_frame(self, w, st):
+    def set_window(self, w):
         if w != self.window:  # a fresh zero buffer; the index is kept
             self.buf[:] = 0.0
             self.bar[:] = BAR_FLOOR
-            # the one documented divergence (dp_engine.cu:run_one): an index beyond the new buffer, an IndexError in the reference,
-            # restarts the cycle
+            # the one documented divergence (dp_engine.cu:TargetSchedule::index_at): an index beyond the new buffer, an IndexError in
+            # the reference, restarts the cycle
             self.idx[self.idx > w] = 0
             self.window = w
+
+    def before_frame(self, w, st):
+        self.set_window(w)
         need = self.track[self.idx[self.track] == 0]
         if need.size:
             rings = (st["latent_buf"][need], st["disp_buf"][need], st["height_buf"][need])
@@ -226,6 +229,12 @@ def _teacher_forced(eng, tm, wl, windows, track, events=None, label=""):
     return bk
 
 
+def _predict_targets(eng, bk, w):
+    """predict_targets at another window: the same window change as a frame at w, before that frame."""
+    eng.predict_targets(w)
+    bk.set_window(w)
+
+
 def _cycles(w, n):
     """`n` predictor calls at window w, the first at frame 0."""
     return [w] * ((n - 1) * max(w, 1) + 1)
@@ -246,6 +255,8 @@ for _pp, _name in ((0, "tc"), (1, "fp32")):
                                                       restarts={5: [2, 9, 17, 30], 11: [9, 21, 36]})
     SCENARIOS[f"restart-lookahead-{_name}"] = dict(n=37, windows=[0] * 13, pred_path=_pp, restarts={6: [1, 5, 36]})
     SCENARIOS[f"restart-boundary-{_name}"] = dict(n=37, windows=[16] * 34, pred_path=_pp, restarts={16: [0, 7, 8]})
+# predict_targets(4) at index 11 of window 16 (beyond the new buffer): the frames at window 4 start at index 0
+SCENARIOS["predict-targets-window-change"] = dict(n=37, windows=[16] * 11 + [4] * 9, predict_targets={11: 4})
 SCENARIOS["set-ring-buffers"] = dict(n=37, windows=_cycles(16, 4), replace_rings=(14, 37))  # after the early call; mid-window
 SCENARIOS["sharp-w0"] = dict(n=37, windows=[0] * 10, model="sharp")
 SCENARIOS["sharp-w16"] = dict(n=37, windows=_cycles(16, 3), model="sharp")
@@ -269,6 +280,8 @@ def test_teacher_forced_frames_vs_float64_bookkeeping(pose_model, model_npz, tem
         events[f] = lambda eng, bk, clips=np.array(clips), w=windows[f]: _restart(eng, bk, clips, rng, w, boundary)
     for f in sc.get("replace_rings", ()):
         events[f] = lambda eng, bk: _replace_rings(eng, bk, rng)
+    for f, w in sc.get("predict_targets", {}).items():
+        events[f] = lambda eng, bk, w=w: _predict_targets(eng, bk, w)
     eng = _engine(pose_model, model_npz, tm, max(64, n))
     try:
         eng.set_predictor_path(sc.get("pred_path", 0))
