@@ -36,6 +36,24 @@ class RunParams(C.Structure):
     ]
 
 
+class ClipSettings(C.Structure):
+    _fields_ = [
+        ("stop_eps_pos", C.c_double),
+        ("stop_eps_rot", C.c_double),
+        ("min_loss_incr", C.c_double),
+        ("max_iter", C.c_int32),
+        ("learning_rate", C.c_float),
+        ("lambda_rot", C.c_float),
+        ("lambda_temporal", C.c_float),
+        ("joint_adjust_joint", C.c_int32),
+        ("joint_adjust_slot", C.c_int32),
+        ("joint_adjust_weight", C.c_float),
+    ]
+
+
+MAX_CLIP_SETTINGS = 32  # DP_MAX_CLIP_SETTINGS
+
+
 class EncoderModelC(C.Structure):
     _fields_ = [(n, c_float_p) for n in ("A0", "b0", "A1", "b1", "A2", "b2", "mu_w", "mu_b", "logvar_w", "logvar_b")]
 
@@ -84,6 +102,7 @@ SIGNATURES = {
     "dp_engine_restart_clips": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
     "dp_engine_get_clip_index": (C.c_int, [_VP, C.c_int, _VP]),
     "dp_engine_frames_to_boundary": (C.c_int, [_VP, C.c_int]),
+    "dp_engine_set_clip_settings": (C.c_int, [_VP, C.c_int, _VP, _VP]),
 }
 
 _lib = None

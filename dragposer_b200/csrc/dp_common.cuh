@@ -75,6 +75,24 @@ struct __align__(16) DpModelImageTC {
 #define DP_TC_TMEM_WORDS 352
 static_assert(sizeof(DpModelImageTC) % 16 == 0, "bulk copy needs a multiple of 16 bytes");
 
+// A clip's optimiser settings (dp_clip_settings, include/dp_engine.h) with the Adam step table of its learning rate.  With a
+// per-clip table the tcgen05 kernel copies each clip's entry to shared memory once per frame and reads it from there: the kernel has
+// no registers to spare for three doubles per clip.
+struct DpClipSetting {
+  double eps_pos, eps_rot, min_incr;
+  const float* adam_tab;  // [2][max_iter]: lr/(1-b1^k), 1/sqrt(1-b2^k), k = 1..max_iter; readable up to index max_iter + the
+                          // launch's max_iter (per-clip tables are padded: a stopped clip's warp still reads them, unused)
+  int max_iter;
+  float lambda_rot, lambda_t;
+  int adj_joint, adj_slot;
+  float adj_w;
+};
+static_assert(sizeof(DpClipSetting) == 56, "copied as seven 8-byte words");
+// lanes 0..6 of a warp copy the entry; the caller synchronises the warp before another lane reads it
+__device__ __forceinline__ void copy_clip_setting(DpClipSetting* dst, const DpClipSetting* src, int lane) {
+  if (lane < (int)(sizeof(DpClipSetting) / 8)) reinterpret_cast<uint2*>(dst)[lane] = reinterpret_cast<const uint2*>(src)[lane];
+}
+
 struct DpFrameArgs {
   const DpModelImage* model;
   const DpModelImageTC* model_tc;    // tables of the tcgen05 kernel
@@ -100,13 +118,16 @@ struct DpFrameArgs {
   const float* tgt_rot;
   int ee_stride;
   int targets_world;  // tgt_pos is world-absolute: subtract the clip's current global position when loading it
-  // optimiser
-  double eps_pos, eps_rot, min_incr;
-  int max_iter;
-  float lambda_rot, lambda_t;
-  int adj_joint, adj_slot;
-  float adj_w;
-  const float* adam_tab;  // [2][max_iter]: lr/(1-b1^k), sqrt(1-b2^k), k = 1..max_iter
+  // optimiser: every clip runs with `uniform` (settings null), or, tcgen05 kernel only, clip c with settings[clip_setting[c]]
+  // (settings[0] when clip_setting is null).  The two cases are separate instantiations of the tcgen05 kernel: reading a per-clip
+  // entry from shared memory puts a load in front of the Adam step's table reads and its stop test, which measured 0.956 against
+  // 0.920 ms per frame at 4 096 clips (DESIGN.md section 3.4); the uniform instantiation reads `uniform` from the kernel parameters.
+  // The fp32 kernel runs a table as one launch per setting, each with that setting as `uniform` over compact copies of its clips.
+  DpClipSetting uniform;
+  const DpClipSetting* settings;
+  const int32_t* clip_setting;
+  int max_iter;      // loop bound: the largest max_iter of the settings in use
+  int fixed_iters;   // every setting in use runs a fixed number of iterations (negative thresholds, min_incr = -inf)
   // outputs
   float* out_pose;    // (B,88), or the packed rows (B,92) = [pose 88 | global_pos 3 | pad] with out_gpos = out_pose + 88
   float* out_gpos;    // (B,3)

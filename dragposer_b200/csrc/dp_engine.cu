@@ -112,6 +112,17 @@ struct dp_engine {
   float* d_adam = nullptr;
   int adam_iters = 0;
   float adam_lr = -1.0f;
+  // Per-clip settings (dp_engine_set_clip_settings).  Without them (settings empty) every clip runs with the frame's dp_run_params.
+  std::vector<dp_clip_settings> settings;  // empty = none
+  std::vector<char> setting_used;          // settings[s] is some clip's setting
+  std::vector<int32_t> clip_setting;       // (n_clips) index of each clip's setting
+  std::vector<DpClipSetting> settings_dev;  // the entries as the kernels read them
+  std::vector<int> group_setting, group_start;  // settings in use; the clips of group_setting[g] are d_group_ids[group_start[g] ..]
+  int settings_max_iter = 0, settings_fixed = 0;  // over the settings in use: largest max_iter, all fixed-iteration
+  unsigned char* d_settings_blk = nullptr;  // device block of the table (dp_engine_set_clip_settings), pointed into by:
+  DpClipSetting* d_settings = nullptr;      // (n_settings)
+  int32_t* d_clip_setting = nullptr;        // (n_clips) each clip's setting
+  int32_t* d_group_ids = nullptr;           // (n_clips) clip ids grouped by setting, ascending within a group
   TpWork tw{};
   // staging for the host-pointer path
   // double-buffered staging of dp_engine_run_frames_host: one contiguous block per slot and direction
@@ -136,6 +147,10 @@ struct dp_engine {
   bool restart_pending = false;
   // compact inputs and outputs of the subset predictor (allocated on first use, max_clips rows)
   float *d_sub_latent = nullptr, *d_sub_disp = nullptr, *d_sub_height = nullptr, *d_sub_target = nullptr;
+  // compact per-clip arrays of the fp32 kernel's per-setting batches (run_fp32_by_setting; allocated on first use, max_clips rows)
+  float* d_sub_frame = nullptr;
+  float* d_sub_trace = nullptr;
+  int sub_trace_iters = 0;
 };
 
 extern "C" const char* dp_engine_last_error(void) { return g_err.c_str(); }
@@ -231,6 +246,7 @@ extern "C" int dp_engine_destroy(dp_engine* e) {
   cudaFree(e->d_latent); cudaFree(e->d_gpos); cudaFree(e->d_grot); cudaFree(e->d_latent_buf);
   cudaFree(e->d_disp_buf); cudaFree(e->d_height_buf); cudaFree(e->d_target_buf); cudaFree(e->d_target_pre); cudaFree(e->d_iters);
   cudaFree(e->d_losses); cudaFree(e->d_trace); cudaFree(e->d_adam); cudaFree(e->d_phase);
+  cudaFree(e->d_settings_blk); cudaFree(e->d_sub_frame); cudaFree(e->d_sub_trace);
   cudaFree(e->tw.enc); cudaFree(e->tw.enc2); cudaFree(e->tw.dec); cudaFree(e->tw.dec2); cudaFree(e->tw.dec_lat); cudaFree(e->tw.ffpart);
   if (e->tw.st_extra) { cudaStreamSynchronize(e->tw.st_extra); cudaStreamDestroy(e->tw.st_extra); }
   if (e->tw.ev_join) cudaEventDestroy(e->tw.ev_join);
@@ -432,6 +448,7 @@ extern "C" int dp_engine_init_clips(dp_engine* e, int n, const float* latent0, c
   e->n_clips = n;
   e->ring_head = 0;
   e->sched.reset(n);
+  e->settings.clear();  // a new batch starts without per-clip settings
   return DP_OK;
 }
 
@@ -443,15 +460,19 @@ extern "C" int dp_engine_set_global_pos(dp_engine* e, int first, int n, const fl
   return DP_OK;
 }
 
-static int ensure_adam(dp_engine* e, int max_iter, float lr) {
-  if (e->d_adam && e->adam_iters == max_iter && e->adam_lr == lr) return DP_OK;
-  // torch/optim/adam.py:414-547: step_size = lr / (1 - beta1^k), sqrt(1 - beta2^k) -- Python doubles
-  std::vector<float> tab(2 * (size_t)max_iter);
+// torch/optim/adam.py:414-547: step_size = lr / (1 - beta1^k), sqrt(1 - beta2^k) -- Python doubles; tab is [2][max_iter]
+static void adam_table(int max_iter, float lr, float* tab) {
   const double lrd = (double)lr;
   for (int k = 1; k <= max_iter; ++k) {
     tab[k - 1] = (float)(lrd / (1.0 - std::pow(0.9, (double)k)));
     tab[max_iter + k - 1] = (float)(1.0 / std::pow(1.0 - std::pow(0.999, (double)k), 0.5));  // kernels multiply by the reciprocal
   }
+}
+
+static int ensure_adam(dp_engine* e, int max_iter, float lr) {
+  if (e->d_adam && e->adam_iters == max_iter && e->adam_lr == lr) return DP_OK;
+  std::vector<float> tab(2 * (size_t)max_iter);
+  adam_table(max_iter, lr, tab.data());
   // earlier frames may still be reading the table on a caller-supplied stream (run_frames_device): settle the whole device first
   CK(cudaDeviceSynchronize());
   if (e->adam_iters != max_iter) {
@@ -467,14 +488,37 @@ static int ensure_adam(dp_engine* e, int max_iter, float lr) {
   return DP_OK;
 }
 
+static dp_clip_settings clip_settings_of(const dp_run_params* p) {
+  return {p->stop_eps_pos, p->stop_eps_rot, p->min_loss_incr, p->max_iter, p->learning_rate, p->lambda_rot, p->lambda_temporal,
+          p->joint_adjust_joint, p->joint_adjust_slot, p->joint_adjust_weight};
+}
+// negative stop thresholds and min_loss_incr = -inf: every iteration runs (the tcgen05 kernel then skips most loss sums)
+static bool fixed_iterations(const dp_clip_settings& s) { return s.stop_eps_pos < 0.0 && s.stop_eps_rot < 0.0 && s.min_loss_incr < -1.7e308; }
+static DpClipSetting device_setting(const dp_clip_settings& s, const float* adam_tab) {
+  return {s.stop_eps_pos, s.stop_eps_rot, s.min_loss_incr, adam_tab, s.max_iter, s.lambda_rot, s.lambda_temporal,
+          s.joint_adjust_joint, s.joint_adjust_slot, s.joint_adjust_weight};
+}
+// the per-clip fields; ee_stride 0 = not known yet (dp_engine_set_clip_settings: each frame checks the slot against its own)
+static int check_setting(const dp_clip_settings& s, int ee_stride) {
+  if (s.max_iter < 1 || s.max_iter > DP_MAX_ITER) return fail(DP_ERR_ARG, "max_iter out of range");
+  if (s.joint_adjust_joint >= DP_JOINTS ||
+      (s.joint_adjust_joint >= 0 && (s.joint_adjust_slot < 0 || (ee_stride && s.joint_adjust_slot >= ee_stride))))
+    return fail(DP_ERR_ARG, "joint adjustment indices out of range");
+  return DP_OK;
+}
+
 static int check_params(const dp_engine* e, const dp_run_params* p, int ee_stride) {
   if (!e->has_pose) return fail(DP_ERR_STATE, "pose model not set");
   if (e->n_clips <= 0) return fail(DP_ERR_STATE, "no clips initialised");
-  if (p->max_iter < 1 || p->max_iter > DP_MAX_ITER) return fail(DP_ERR_ARG, "max_iter out of range");
   if (int rc = check_window(p->temporal_future_window)) return rc;
   if (ee_stride < 1 || ee_stride > DP_JOINTS) return fail(DP_ERR_ARG, "ee_stride out of range");
-  if (p->joint_adjust_joint >= DP_JOINTS || (p->joint_adjust_joint >= 0 && (p->joint_adjust_slot < 0 || p->joint_adjust_slot >= ee_stride)))
-    return fail(DP_ERR_ARG, "joint adjustment indices out of range");
+  if (e->settings.empty()) {
+    if (int rc = check_setting(clip_settings_of(p), ee_stride)) return rc;
+  } else {
+    for (size_t s = 0; s < e->settings.size(); ++s)
+      if (e->setting_used[s])
+        if (int rc = check_setting(e->settings[s], ee_stride)) return rc;
+  }
   if (p->extension_losses < 0 || p->extension_losses > 15) return fail(DP_ERR_ARG, "extension_losses must be a mask of DP_EXT_* bits");
   if (p->extension_losses && p->decoder_path == 3)
     return fail(DP_ERR_UNSUPPORTED, "the extension losses run on the fp32 CUDA-core frame kernel: use decoder_path 0 or 1");
@@ -483,13 +527,103 @@ static int check_params(const dp_engine* e, const dp_run_params* p, int ee_strid
   return DP_OK;
 }
 
-// host-side tracker counts: 1 <= n_ee[c] <= ee_stride, and the joint-adjustment slot must be an active tracker of every clip
-static int check_n_ee(const int32_t* n_ee, size_t count, int ee_stride, const dp_run_params* p) {
+// host-side tracker counts: 1 <= n_ee[i] <= ee_stride, and a clip's joint-adjustment slot must be one of its active trackers.
+// Entry i belongs to clip i % n_clips, whose setting is the frame's (p) or its own (user table); no engine: no joint adjustment.
+static int check_n_ee(const dp_engine* e, const dp_run_params* p, const int32_t* n_ee, size_t count, int ee_stride) {
   if (!n_ee) return DP_OK;
-  const int need = (p && p->joint_adjust_joint >= 0) ? p->joint_adjust_slot + 1 : 1;
-  for (size_t i = 0; i < count; ++i)
-    if (n_ee[i] < need || n_ee[i] > ee_stride)
-      return fail(DP_ERR_ARG, "n_ee entries must lie in [1, ee_stride] and cover the joint-adjustment slot");
+  auto need = [](const dp_clip_settings& s) { return s.joint_adjust_joint >= 0 ? s.joint_adjust_slot + 1 : 1; };
+  const bool table = e && !e->settings.empty();
+  int need_of[DP_MAX_CLIP_SETTINGS];
+  for (size_t s = 0; table && s < e->settings.size(); ++s) need_of[s] = need(e->settings[s]);
+  const int need_all = e && !table ? need(clip_settings_of(p)) : 1;
+  for (size_t i = 0; i < count; ++i) {
+    const int nd = table ? need_of[e->clip_setting[i % e->clip_setting.size()]] : need_all;
+    if (n_ee[i] < nd || n_ee[i] > ee_stride)
+      return fail(DP_ERR_ARG, "n_ee entries must lie in [1, ee_stride] and cover the clip's joint-adjustment slot");
+  }
+  return DP_OK;
+}
+
+// The Adam table of the frames of one call: dp_run_params' (ensure_adam), unless per-clip settings bring their own.
+static int prepare_settings(dp_engine* e, const dp_run_params* p) {
+  return e->settings.empty() ? ensure_adam(e, p->max_iter, p->learning_rate) : DP_OK;
+}
+
+extern "C" int dp_engine_set_clip_settings(dp_engine* e, int n, const dp_clip_settings* settings, const int32_t* clip_setting) {
+  if (!e) return fail(DP_ERR_ARG, "null engine");
+  if (n < 0 || n > DP_MAX_CLIP_SETTINGS) return fail(DP_ERR_ARG, "dp_engine_set_clip_settings: n_settings must lie in [0, DP_MAX_CLIP_SETTINGS]");
+  if (n == 0) {
+    e->settings.clear();
+    return DP_OK;
+  }
+  if (!settings) return fail(DP_ERR_ARG, "dp_engine_set_clip_settings: null argument");
+  if (e->n_clips <= 0) return fail(DP_ERR_STATE, "dp_engine_set_clip_settings: no clips initialised (dp_engine_init_clips)");
+  const int B = e->n_clips;
+  std::vector<int32_t> idx(B, 0);
+  if (clip_setting) idx.assign(clip_setting, clip_setting + B);
+  std::vector<char> used(n, 0);
+  for (int c = 0; c < B; ++c) {
+    if (idx[c] < 0 || idx[c] >= n) return fail(DP_ERR_ARG, "dp_engine_set_clip_settings: clip setting index out of range");
+    used[idx[c]] = 1;
+  }
+  for (int s = 0; s < n; ++s)
+    if (int rc = check_setting(settings[s], 0)) return rc;
+  // One device block, replaced as a whole: the entries (n), each clip's index (B), the clips of each setting in use in ascending order
+  // (B; the fp32 kernel runs one launch per setting over them), and one Adam table per setting, built with the expressions of
+  // ensure_adam so that a clip's steps are bitwise a uniform run's.  Each table is [2][max_iter] inside a block of 2 x the largest
+  // max_iter of the table: the tcgen05 kernel's warps keep reading their clips' tables after the clips stopped, up to the loop's end.
+  int stride = 0, max_iter = 0, fixed = 1;
+  for (int s = 0; s < n; ++s) {
+    stride = std::max(stride, (int)settings[s].max_iter);
+    if (used[s]) {
+      max_iter = std::max(max_iter, (int)settings[s].max_iter);
+      fixed = fixed && fixed_iterations(settings[s]);
+    }
+  }
+  std::vector<int> group_setting, group_start(1, 0);
+  std::vector<int32_t> group_ids;
+  for (int s = 0; s < n; ++s) {
+    if (!used[s]) continue;
+    for (int c = 0; c < B; ++c)
+      if (idx[c] == s) group_ids.push_back(c);
+    group_setting.push_back(s);
+    group_start.push_back((int)group_ids.size());
+  }
+  const size_t ids_off = (size_t)n * sizeof(DpClipSetting), group_off = ids_off + (size_t)B * 4;
+  const size_t tab_off = (group_off + (size_t)B * 4 + 15) & ~size_t(15), bytes = tab_off + (size_t)n * 2 * stride * 4;
+  std::vector<unsigned char> blk(bytes, 0);
+  CK(cudaSetDevice(e->device));
+  unsigned char* d_blk = nullptr;
+  CK(cudaMalloc(&d_blk, bytes));
+  std::vector<DpClipSetting> dev(n);
+  for (int s = 0; s < n; ++s) {
+    float* tab = reinterpret_cast<float*>(blk.data() + tab_off) + (size_t)s * 2 * stride;
+    adam_table(settings[s].max_iter, settings[s].learning_rate, tab);
+    dev[s] = device_setting(settings[s], reinterpret_cast<const float*>(d_blk + tab_off) + (size_t)s * 2 * stride);
+  }
+  memcpy(blk.data(), dev.data(), ids_off);
+  memcpy(blk.data() + ids_off, idx.data(), (size_t)B * 4);
+  memcpy(blk.data() + group_off, group_ids.data(), (size_t)B * 4);
+  // frames in flight, on any stream, may still read the block being replaced
+  cudaError_t err = cudaDeviceSynchronize();
+  if (err == cudaSuccess) err = cudaMemcpy(d_blk, blk.data(), bytes, cudaMemcpyHostToDevice);
+  if (err != cudaSuccess) {
+    cudaFree(d_blk);
+    return fail(DP_ERR_CUDA, std::string("dp_engine_set_clip_settings: ") + cudaGetErrorString(err));
+  }
+  cudaFree(e->d_settings_blk);
+  e->d_settings_blk = d_blk;
+  e->d_settings = reinterpret_cast<DpClipSetting*>(d_blk);
+  e->d_clip_setting = reinterpret_cast<int32_t*>(d_blk + ids_off);
+  e->d_group_ids = reinterpret_cast<int32_t*>(d_blk + group_off);
+  e->settings.assign(settings, settings + n);
+  e->settings_dev = dev;
+  e->setting_used = used;
+  e->clip_setting = idx;
+  e->group_setting = group_setting;
+  e->group_start = group_start;
+  e->settings_max_iter = max_iter;
+  e->settings_fixed = fixed;
   return DP_OK;
 }
 
@@ -531,6 +665,86 @@ static int set_window(dp_engine* e, int W, cudaStream_t st) {
   CK(cudaMemsetAsync(e->d_target_buf, 0, (size_t)e->n_clips * (W + 1) * DP_L * 4, st));
   e->sched.current_index = e->sched.index_at(W);
   e->sched.target_rows = W + 1;
+  return DP_OK;
+}
+
+// Per-clip settings on the fp32 frame kernel.  Its no-table code runs each setting's clips as a batch of their own: their rows are
+// gathered into compact arrays, the kernel runs on those with the setting as its uniform parameters, and the results are scattered
+// back.  So a clip computes exactly what a batch of only its setting's clips computes: the same instantiation on the same warp
+// positions.  (A second instantiation that reads per-clip settings, or indexes clips through a list, compiles the same arithmetic
+// with other multiply-add pairings and differs in the last bits.)
+static int run_fp32_by_setting(dp_engine* e, const DpFrameArgs& a, cudaStream_t st) {
+  const size_t M = (size_t)e->max_clips;
+  constexpr int kWords = DP_L + 3 + 4 + DP_L + 1 + DP_JOINTS * 15 + DP_PAST * (DP_L + 3 + DP_NH) + DP_ROW + 3 + 1 + 3;
+  if (!e->d_sub_frame) CK(cudaMalloc(&e->d_sub_frame, M * kWords * 4));
+  if (a.trace && e->sub_trace_iters < a.trace_iters) {
+    cudaFree(e->d_sub_trace);
+    e->d_sub_trace = nullptr;
+    CK(cudaMalloc(&e->d_sub_trace, M * a.trace_iters * 52 * 4));
+    e->sub_trace_iters = a.trace_iters;
+  }
+  float* next = e->d_sub_frame;
+  auto take = [&](int w) { float* r = next; next += M * w; return r; };
+  float *c_lat = take(DP_L), *c_gpos = take(3), *c_grot = take(4), *c_tgt = take(DP_L), *c_nee = take(1), *c_j = take(DP_JOINTS);
+  float *c_w = take(2 * DP_JOINTS), *c_tp = take(3 * DP_JOINTS), *c_tr = take(9 * DP_JOINTS), *c_lb = take(DP_PAST * DP_L);
+  float *c_db = take(DP_PAST * 3), *c_hb = take(DP_PAST * DP_NH), *c_out = take(DP_ROW), *c_og = take(3), *c_it = take(1), *c_ls = take(3);
+  const int S = a.ee_stride, head = a.ring_head;
+  const bool packed = a.out_pose_stride == DP_ROW;
+  DpRowCopies in{}, out{};
+  auto add = [](DpRowCopies& c, const void* src, void* dst, int width, int src_stride, int dst_stride) {
+    c.c[c.n++] = DpRowCopy{reinterpret_cast<const float*>(src), reinterpret_cast<float*>(dst), width, src_stride, dst_stride};
+  };
+  add(in, a.latent, c_lat, DP_L, DP_L, DP_L);
+  add(in, a.gpos, c_gpos, 3, 3, 3);
+  add(in, a.grot, c_grot, 4, 4, 4);
+  add(in, a.target_buf + (size_t)a.target_index * DP_L, c_tgt, DP_L, a.target_rows * DP_L, DP_L);
+  if (a.n_ee) add(in, a.n_ee, c_nee, 1, 1, 1);
+  if (!a.shared_trackers) {
+    add(in, a.joints, c_j, S, S, S);
+    add(in, a.weights, c_w, 2 * S, 2 * S, 2 * S);
+  }
+  add(in, a.tgt_pos, c_tp, 3 * S, 3 * S, 3 * S);
+  add(in, a.tgt_rot, c_tr, 9 * S, 9 * S, 9 * S);
+  add(out, c_lat, a.latent, DP_L, DP_L, DP_L);
+  add(out, c_gpos, a.gpos, 3, 3, 3);
+  add(out, c_grot, a.grot, 4, 4, 4);
+  add(out, c_lb + head * DP_L, a.latent_buf + head * DP_L, DP_L, DP_PAST * DP_L, DP_PAST * DP_L);
+  add(out, c_db + head * 3, a.disp_buf + head * 3, 3, DP_PAST * 3, DP_PAST * 3);
+  add(out, c_hb + head * DP_NH, a.height_buf + head * DP_NH, DP_NH, DP_PAST * DP_NH, DP_PAST * DP_NH);
+  if (packed) {
+    add(out, c_out, a.out_pose, DP_POSE + 3, DP_ROW, DP_ROW);  // the pad word stays the caller's
+  } else {
+    add(out, c_out, a.out_pose, DP_POSE, DP_POSE, DP_POSE);
+    add(out, c_og, a.out_gpos, 3, 3, 3);
+  }
+  add(out, c_it, a.out_iters, 1, 1, 1);
+  add(out, c_ls, a.out_losses, 3, 3, 3);
+  if (a.trace) add(out, e->d_sub_trace, a.trace, a.trace_iters * 52, a.trace_iters * 52, a.trace_iters * 52);
+  for (size_t g = 0; g < e->group_setting.size(); ++g) {
+    const int s = e->group_setting[g], n = e->group_start[g + 1] - e->group_start[g];
+    const int32_t* ids = e->d_group_ids + e->group_start[g];
+    DpFrameArgs b = a;
+    b.settings = nullptr;
+    b.clip_setting = nullptr;
+    b.uniform = e->settings_dev[s];
+    b.max_iter = e->settings[s].max_iter;
+    b.n_clips = n;
+    b.latent = c_lat; b.gpos = c_gpos; b.grot = c_grot;
+    b.target_buf = c_tgt; b.target_rows = 1; b.target_index = 0;
+    b.n_ee = a.n_ee ? reinterpret_cast<const int32_t*>(c_nee) : nullptr;
+    if (!a.shared_trackers) { b.joints = reinterpret_cast<const int32_t*>(c_j); b.weights = c_w; }
+    b.tgt_pos = c_tp; b.tgt_rot = c_tr;
+    b.latent_buf = c_lb; b.disp_buf = c_db; b.height_buf = c_hb;
+    b.out_pose = c_out; b.out_gpos = packed ? c_out + DP_POSE : c_og;
+    b.out_iters = reinterpret_cast<int32_t*>(c_it); b.out_losses = c_ls;
+    b.trace = a.trace ? e->d_sub_trace : nullptr;
+    CK(dp_copy_rows_launch(in, ids, n, 0, st));
+    // the kernel writes trace rows of active iterations only: the compact rows still hold the previous setting's
+    if (a.trace) CK(cudaMemsetAsync(e->d_sub_trace, 0, (size_t)n * a.trace_iters * 52 * 4, st));
+    CK(dp_frame_simt_launch(b, e->num_sms, st));
+    CK(dp_copy_rows_launch(out, ids, n, 1, st));
+    e->launches += 3;
+  }
   return DP_OK;
 }
 
@@ -585,11 +799,21 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
     }
     a.target_buf = e->d_target_buf; a.target_rows = W + 1; a.target_index = g;
   }
-  if (e->trace_enabled && (!e->d_trace || e->trace_iters < p->max_iter)) {
+  if (e->settings.empty()) {
+    a.uniform = device_setting(clip_settings_of(p), e->d_adam);
+    a.max_iter = p->max_iter;
+    a.fixed_iters = fixed_iterations(clip_settings_of(p));
+  } else {
+    a.settings = e->d_settings;
+    a.clip_setting = e->d_clip_setting;
+    a.max_iter = e->settings_max_iter;
+    a.fixed_iters = e->settings_fixed;
+  }
+  if (e->trace_enabled && (!e->d_trace || e->trace_iters < a.max_iter)) {
     cudaFree(e->d_trace);
     e->d_trace = nullptr;
-    CK(cudaMalloc(&e->d_trace, (size_t)e->max_clips * p->max_iter * 52 * 4));
-    e->trace_iters = p->max_iter;
+    CK(cudaMalloc(&e->d_trace, (size_t)e->max_clips * a.max_iter * 52 * 4));
+    e->trace_iters = a.max_iter;
   }
   if (e->trace_enabled) CK(cudaMemsetAsync(e->d_trace, 0, (size_t)e->max_clips * e->trace_iters * 52 * 4, st));
   a.model = e->d_model;
@@ -602,11 +826,6 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
   a.n_ee = n_ee; a.joints = joints; a.weights = weights; a.shared_trackers = shared;
   a.tgt_pos = tgt_pos; a.tgt_rot = tgt_rot; a.ee_stride = ee_stride;
   a.targets_world = p->targets_world ? 1 : 0;
-  a.eps_pos = p->stop_eps_pos; a.eps_rot = p->stop_eps_rot; a.min_incr = p->min_loss_incr;
-  a.max_iter = p->max_iter;
-  a.lambda_rot = p->lambda_rot; a.lambda_t = p->lambda_temporal;
-  a.adj_joint = p->joint_adjust_joint; a.adj_slot = p->joint_adjust_slot; a.adj_w = p->joint_adjust_weight;
-  a.adam_tab = e->d_adam;
   a.out_pose = out_pose; a.out_iters = e->d_iters; a.out_losses = e->d_losses;
   if (out_gpos) { a.out_gpos = out_gpos; a.out_pose_stride = DP_POSE; a.out_gpos_stride = 3; }
   else { a.out_gpos = out_pose + DP_POSE; a.out_pose_stride = a.out_gpos_stride = DP_ROW; }  // packed wire rows
@@ -619,10 +838,16 @@ static int run_one(dp_engine* e, const dp_run_params* p, const int32_t* n_ee, co
   a.ext_mask = p->extension_losses;
   a.floor_level = p->floor_level;
   const int path = p->extension_losses ? 1 : (p->decoder_path ? p->decoder_path : (e->n_clips >= 512 ? 3 : 1));
-  if (path == 3) CK(dp_frame_tc16_launch(a, e->num_sms, st));
-  else CK(dp_frame_simt_launch(a, e->num_sms, st));
+  if (path == 3) {
+    CK(dp_frame_tc16_launch(a, e->num_sms, st));
+    ++e->launches;
+  } else if (!a.settings) {
+    CK(dp_frame_simt_launch(a, e->num_sms, st));
+    ++e->launches;
+  } else {
+    if (int rc2 = run_fp32_by_setting(e, a, st)) return rc2;
+  }
   e->last_path = path;
-  ++e->launches;
   if (e->profiling) {
     CK(cudaEventRecord(ev[2], st));
     for (int i = 0; i < 3; ++i) e->prof_events.push_back(ev[i]);
@@ -641,7 +866,7 @@ extern "C" int dp_engine_run_frames_device(dp_engine* e, const dp_run_params* p,
   if (rc) return rc;
   CK(cudaSetDevice(e->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-  rc = ensure_adam(e, p->max_iter, p->learning_rate);
+  rc = prepare_settings(e, p);
   if (rc) return rc;
   const size_t B = (size_t)e->n_clips, S = (size_t)ee_stride;
   for (int f = 0; f < n_frames; ++f) {
@@ -702,7 +927,7 @@ extern "C" int dp_engine_run_frame_host(dp_engine* e, const dp_run_params* p, co
   CK(cudaSetDevice(e->device));
   rc = ensure_pipe(e, ee_stride);
   if (rc) return rc;
-  rc = ensure_adam(e, p->max_iter, p->learning_rate);
+  rc = prepare_settings(e, p);
   if (rc) return rc;
   // one contiguous pinned block in, one out: a single copy each way (this is the B = 1 latency path of the DLL)
   dp_engine::FramePipe& P = e->pipe;
@@ -711,7 +936,7 @@ extern "C" int dp_engine_run_frame_host(dp_engine* e, const dp_run_params* p, co
   const size_t nj = shared ? S : B * S;
   const PipeLayout L((size_t)e->max_clips, (size_t)P.stride);
   unsigned char* h = P.h_in[0];
-  if ((rc = check_n_ee(n_ee, B, ee_stride, p)) != DP_OK) return rc;
+  if ((rc = check_n_ee(e, p, n_ee, B, ee_stride)) != DP_OK) return rc;
   if (n_ee) memcpy(h + L.nee, n_ee, B * 4);
   memcpy(h + L.joints, joints, nj * 4);
   memcpy(h + L.w, weights, nj * 8);
@@ -743,8 +968,8 @@ extern "C" int dp_engine_run_frames_host(dp_engine* e, const dp_run_params* p, i
   CK(cudaSetDevice(e->device));
   rc = ensure_pipe(e, ee_stride);
   if (rc) return rc;
-  if ((rc = check_n_ee(n_ee, (size_t)n_frames * (size_t)e->n_clips, ee_stride, p)) != DP_OK) return rc;
-  rc = ensure_adam(e, p->max_iter, p->learning_rate);
+  if ((rc = check_n_ee(e, p, n_ee, (size_t)n_frames * (size_t)e->n_clips, ee_stride)) != DP_OK) return rc;
+  rc = prepare_settings(e, p);
   if (rc) return rc;
   dp_engine::FramePipe& P = e->pipe;
   cudaStream_t st = e->stream;
@@ -906,7 +1131,7 @@ extern "C" int dp_engine_eval_gradient(dp_engine* e, int n, const float* latents
     return fail(DP_ERR_ARG, "dp_engine_eval_gradient: null argument");
   if (!e->has_pose) return fail(DP_ERR_STATE, "pose model not set");
   if (ee_stride < 1 || ee_stride > DP_JOINTS) return fail(DP_ERR_ARG, "ee_stride out of range");
-  if (int rcn = check_n_ee(n_ee, (size_t)n, ee_stride, nullptr)) return rcn;
+  if (int rcn = check_n_ee(nullptr, nullptr, n_ee, (size_t)n, ee_stride)) return rcn;
   if (extension_losses < 0 || extension_losses > 15) return fail(DP_ERR_ARG, "extension_losses must be a mask of DP_EXT_* bits");
   if (extension_losses && decoder_path == 3) return fail(DP_ERR_UNSUPPORTED, "the extension losses run on the fp32 CUDA-core frame kernel");
   CK(cudaSetDevice(e->device));
@@ -938,9 +1163,10 @@ extern "C" int dp_engine_eval_gradient(dp_engine* e, int n, const float* latents
   a.target_buf = d_t; a.target_rows = 1; a.target_index = 0;
   a.n_ee = d_ne; a.joints = d_j; a.weights = d_w; a.shared_trackers = shared; a.tgt_pos = d_tp; a.tgt_rot = d_tr;
   a.ee_stride = ee_stride;
-  a.eps_pos = -1.0; a.eps_rot = -1.0; a.min_incr = -std::numeric_limits<double>::infinity();
-  a.max_iter = 1; a.lambda_rot = lambda_rot; a.lambda_t = lambda_temporal; a.adj_joint = -1;
-  a.adam_tab = d_adam; a.out_losses = d_loss; a.eval_only = 1; a.eval_grad = d_grad; a.eval_pos = d_pos;
+  // one evaluation: no stop rule, no joint adjustment
+  a.uniform = {-1.0, -1.0, -std::numeric_limits<double>::infinity(), d_adam, 1, lambda_rot, lambda_temporal, -1, 0, 0.0f};
+  a.max_iter = 1;
+  a.out_losses = d_loss; a.eval_only = 1; a.eval_grad = d_grad; a.eval_pos = d_pos;
   a.gpos = d_gp; a.ext_mask = extension_losses; a.floor_level = floor_level;
   if (decoder_path == 3) CK(dp_frame_tc16_launch(a, e->num_sms, e->stream));
   else CK(dp_frame_simt_launch(a, e->num_sms, e->stream));

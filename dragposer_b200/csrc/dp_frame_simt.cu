@@ -97,7 +97,7 @@ __global__ void __launch_bounds__(512, 1) dp_frame_simt_kernel(const __grid_cons
     ne = max(1, min(ne, A.ee_stride));
     gpos_y[c] = A.ext_mask ? A.gpos[cc * 3 + 1] : 0.0f;
     inv3e[c] = 1.0f / (3.0f * (float)ne);
-    lrot9e[c] = A.lambda_rot / (9.0f * (float)ne);
+    lrot9e[c] = A.uniform.lambda_rot / (9.0f * (float)ne);
 #pragma unroll
     for (int i = 0; i < 4; ++i) g[c][i] = A.grot[cc * 4 + i];
     z[c] = tl[c] = make_float2(0.f, 0.f);
@@ -142,12 +142,12 @@ __global__ void __launch_bounds__(512, 1) dp_frame_simt_kernel(const __grid_cons
     lp[c] = lr[c] = lt[c] = __int_as_float(0x7f800000);
     iters[c] = 0;
   }
-  const float lt_scale = A.lambda_t * (1.0f / (float)DP_L);
+  const float lt_scale = A.uniform.lambda_t * (1.0f / (float)DP_L);
   for (int it = 0; it < A.max_iter; ++it) {
     bool any = false;
 #pragma unroll
     for (int c = 0; c < CPW; ++c) {
-      active[c] = active[c] && ((double)lp[c] > A.eps_pos || (double)lr[c] > A.eps_rot) && (incr[c] > A.min_incr);
+      active[c] = active[c] && ((double)lp[c] > A.uniform.eps_pos || (double)lr[c] > A.uniform.eps_rot) && (incr[c] > A.uniform.min_incr);
       any = any || active[c];
     }
     if (!any) break;
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(512, 1) dp_frame_simt_kernel(const __grid_cons
     __syncwarp();
     dense_pairs<CPW, DP_H0, DP_L>(M.W0, nullptr, sb, acc, lane);
     // temporal term, loss bookkeeping, Adam (torch/optim/adam.py single-tensor path)
-    const float step_size = A.adam_tab[it], inv_bc2s = A.adam_tab[A.max_iter + it];  // lr/(1-b1^k), 1/sqrt(1-b2^k)
+    const float step_size = A.uniform.adam_tab[it], inv_bc2s = A.uniform.adam_tab[A.max_iter + it];  // lr/(1-b1^k), 1/sqrt(1-b2^k)
 #pragma unroll
     for (int c = 0; c < CPW; ++c) {
       const float dx = z[c].x - tl[c].x, dy = z[c].y - tl[c].y;
@@ -301,12 +301,12 @@ __global__ void __launch_bounds__(512, 1) dp_frame_simt_kernel(const __grid_cons
       p0[i] = __shfl_sync(0xffffffffu, p[i], 0);
       gp[i] = A.gpos[clip * 3 + i] + p0[i];
     }
-    if (A.adj_joint >= 0) {  // joint adjustment (drag_pose.py:374-381)
-      const float* tp = A.tgt_pos + ((size_t)clip * A.ee_stride + A.adj_slot) * 3;
+    if (A.uniform.adj_joint >= 0) {  // joint adjustment (drag_pose.py:374-381)
+      const float* tp = A.tgt_pos + ((size_t)clip * A.ee_stride + A.uniform.adj_slot) * 3;
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
-        const float pj = __shfl_sync(0xffffffffu, p[i], A.adj_joint);
-        adj[i] = ((tp[i] - (A.targets_world ? A.gpos[clip * 3 + i] : 0.0f)) - pj) * A.adj_w;
+        const float pj = __shfl_sync(0xffffffffu, p[i], A.uniform.adj_joint);
+        adj[i] = ((tp[i] - (A.targets_world ? A.gpos[clip * 3 + i] : 0.0f)) - pj) * A.uniform.adj_w;
         gp[i] += adj[i];
       }
     }

@@ -72,6 +72,7 @@ struct SmemT {
   double prev[NC];                                  // previous total loss (early stopping compares in double)
   float loss[NC][3];                                // last evaluated lp, lr, lt
   int iters[NC];
+  DpClipSetting set[NC];                            // optimiser settings of each clip column
   uint64_t bar_w, bar_mma[kGroups];
   uint32_t tmem_base;
   __device__ __forceinline__ const DpModelImageTC& M() const { return *reinterpret_cast<const DpModelImageTC*>(model); }
@@ -244,7 +245,8 @@ __device__ __forceinline__ void tc_layer4(Ctx& c, const unsigned char* src, int 
 }
 
 // CLOCK: the phase clock / timeline of CTA 0 (profiling level 2) is compiled into a second instantiation only
-template <bool CLOCK>
+// TABLE: per-clip settings (DpFrameArgs::settings); otherwise every clip runs with DpFrameArgs::uniform
+template <bool CLOCK, bool TABLE>
 __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __grid_constant__ DpFrameArgs A) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   SmemT& S = *reinterpret_cast<SmemT*>(smem_raw);
@@ -302,8 +304,10 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
     const int cc = valid[c] ? clip : 0;
     int ne = A.n_ee ? A.n_ee[cc] : A.ee_stride;
     ne = max(1, min(ne, A.ee_stride));
+    const DpClipSetting* s = TABLE ? A.settings + (A.clip_setting ? A.clip_setting[cc] : 0) : &A.uniform;
+    if (TABLE) copy_clip_setting(&S.set[n0 + c], s, lane);
     inv3e[c] = 1.0f / (3.0f * (float)ne);
-    lrot9e[c] = A.lambda_rot / (9.0f * (float)ne);
+    lrot9e[c] = s->lambda_rot / (9.0f * (float)ne);
     if (lane < 4) reinterpret_cast<float*>(&S.groot2[warp][lane])[c] = A.grot[cc * 4 + lane];
     if (lane == 0) {
       S.prev[n0 + c] = 10000000.0;
@@ -394,11 +398,13 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
 
   // ---- optimisation loop (drag_pose.py:296-355)
   // early-stop test of the NEXT iteration, evaluated right after each Adam step (initial losses are +inf, initial increment 1)
-  bool active[CPW] = {valid[0] && 1.0 > A.min_incr, valid[1] && 1.0 > A.min_incr};
-  const float lt_scale = A.lambda_t * (1.0f / (float)DP_L);
+  const DpClipSetting& cs0 = TABLE ? S.set[n0] : A.uniform;
+  const DpClipSetting& cs1 = TABLE ? S.set[n0 + 1] : A.uniform;
+  bool active[CPW] = {valid[0] && 1.0 > cs0.min_incr, valid[1] && 1.0 > cs1.min_incr};
   // A fixed number of iterations (negative stop thresholds, min_loss_incr = -inf: the headline workload) looks at the tracker losses
-  // of an iteration only to report the last ones: their warp sums are skipped on the other iterations (dp_fk2.cuh, want_loss)
-  const bool fixed_iters = A.eps_pos < 0.0 && A.eps_rot < 0.0 && A.min_incr < -1.7e308 && !A.trace && !A.eval_only;
+  // of an iteration only to report each clip's last ones: their warp sums are skipped on the other iterations (dp_fk2.cuh,
+  // want_loss).  One setting in use that stops early turns this off for the whole launch.
+  const bool fixed_iters = A.fixed_iters && !A.trace && !A.eval_only;
   const bool clocked = CLOCK && A.phase_cycles != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
   long long tick = clocked ? clock64() : 0;
   auto phase_done = [&](int i) {
@@ -415,9 +421,10 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
   };
   for (int it = 0; it < A.max_iter; ++it) {
     if (!group_or(gid, active[0] || active[1])) break;  // also publishes the latent pieces written by the Adam epilogue
-    if (lane == 0) {  // the Adam epilogue reads two table entries: pull their lines into L1 now instead of stalling there
-      asm volatile("prefetch.global.L1 [%0];" ::"l"(A.adam_tab + it));
-      asm volatile("prefetch.global.L1 [%0];" ::"l"(A.adam_tab + A.max_iter + it));
+    if (TABLE ? lane < CPW : lane == 0) {  // the Adam epilogue reads two table entries per clip: pull their lines into L1 now
+      const DpClipSetting& cs = TABLE ? S.set[n0 + lane] : A.uniform;
+      asm volatile("prefetch.global.L1 [%0];" ::"l"(cs.adam_tab + it));
+      asm volatile("prefetch.global.L1 [%0];" ::"l"(cs.adam_tab + cs.max_iter + it));
     }
     phase_done(3);
     stamp(it, 0);
@@ -429,7 +436,8 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
       // one packed pass; dL/dy leaves it scaled per clip into [16, 32) (exact powers of two, undone when dL/dz is read)
       const FkOut2 o = fk_loss2<true, false, true>(M, lane_idx, &S.y2[warp][0][0], &S.trk2[warp][0][0], &S.groot2[warp][0], &S.fkscr[warp][0],
                                                    inv3e2, lrot9e2, lane, nullptr, nullptr, nullptr, nullptr, &S.bscale[n0],
-                                                   EmitDyPieces{S.dyimg, gid, 2 * wg, lane}, !fixed_iters || it + 1 == A.max_iter);
+                                                   EmitDyPieces{S.dyimg, gid, 2 * wg, lane},
+                                                   !fixed_iters || it + 1 == cs0.max_iter || it + 1 == cs1.max_iter);
       phase_done(4);
       if (active[0]) { nlp[0] = o.lp.v.x; nlr[0] = o.lr.v.x; }
       if (active[1]) { nlp[1] = o.lp.v.y; nlr[1] = o.lr.v.y; }
@@ -461,7 +469,10 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
       const bool lat = lane < DP_L;
       float2 z = make_float2(0.f, 0.f), tl = z, am = z, av = z;
       if (lat) { z = S.st[warp][ST_Z][lane]; tl = S.st[warp][ST_TL][lane]; am = S.st[warp][ST_M][lane]; av = S.st[warp][ST_V][lane]; }
-      const float step_size = A.adam_tab[it], inv_bc2s = A.adam_tab[A.max_iter + it];  // lr/(1-b1^k), 1/sqrt(1-b2^k)
+      // lr/(1-b1^k), 1/sqrt(1-b2^k) of each clip's own table
+      const float step0 = cs0.adam_tab[it], inv_bc2s0 = cs0.adam_tab[cs0.max_iter + it];
+      const float step1 = cs1.adam_tab[it], inv_bc2s1 = cs1.adam_tab[cs1.max_iter + it];
+      const float lt_scale0 = cs0.lambda_t * (1.0f / (float)DP_L), lt_scale1 = cs1.lambda_t * (1.0f / (float)DP_L);
       const float us0 = wsc * S.bscale[n0], us1 = wsc * S.bscale[n0 + 1];               // undo the weight and dL/dy scalings
       const double prev0 = S.prev[n0], prev1 = S.prev[n0 + 1];
       const float dx = z.x - tl.x, dy = z.y - tl.y;
@@ -471,7 +482,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
         s0 += __shfl_xor_sync(0xffffffffu, s0, o);
         s1 += __shfl_xor_sync(0xffffffffu, s1, o);
       }
-      const float nlt0 = s0 * lt_scale, nlt1 = s1 * lt_scale;
+      const float nlt0 = s0 * lt_scale0, nlt1 = s1 * lt_scale1;
       mbar_wait(&S.bar_mma[gid], ctx.phase);
       tc_fence_after();
       float d1[2], d2[2];
@@ -481,7 +492,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
       tmem_ld_wait();
       tc_fence_before();
       ctx.phase ^= 1u;
-      const float gx = fmaf(2.0f * lt_scale, dx, (d1[0] + d2[0]) * us0), gy = fmaf(2.0f * lt_scale, dy, (d1[1] + d2[1]) * us1);
+      const float gx = fmaf(2.0f * lt_scale0, dx, (d1[0] + d2[0]) * us0), gy = fmaf(2.0f * lt_scale1, dy, (d1[1] + d2[1]) * us1);
       if (A.trace && lat) {
         if (active[0]) {
           float* row = A.trace + ((size_t)clip0 * A.trace_iters + it) * 52;
@@ -503,8 +514,8 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
         const float mx = fmaf(0.1f, gx - am.x, am.x), my = fmaf(0.1f, gy - am.y, am.y);
         const float vx = av.x * 0.999f + (0.001f * gx) * gx, vy = av.y * 0.999f + (0.001f * gy) * gy;
         // MUFU square root / reciprocal without the denormal range extension: a denormal second moment is far below eps = 1e-8
-        const float ux = (-step_size * mx) * rcp_ftz(fmaf(sqrt_ftz(vx), inv_bc2s, 1e-8f));
-        const float uy = (-step_size * my) * rcp_ftz(fmaf(sqrt_ftz(vy), inv_bc2s, 1e-8f));
+        const float ux = (-step0 * mx) * rcp_ftz(fmaf(sqrt_ftz(vx), inv_bc2s0, 1e-8f));
+        const float uy = (-step1 * my) * rcp_ftz(fmaf(sqrt_ftz(vy), inv_bc2s1, 1e-8f));
         const bool a0 = active[0], a1 = active[1];
         S.st[warp][ST_M][lane] = make_float2(a0 ? mx : am.x, a1 ? my : am.y);
         S.st[warp][ST_V][lane] = make_float2(a0 ? vx : av.x, a1 ? vy : av.y);
@@ -532,8 +543,8 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
           S.iters[n0 + 1] += 1;
         }
       }
-      active[0] = active[0] && ((double)nlp[0] > A.eps_pos || (double)nlr[0] > A.eps_rot) && (incr0 > A.min_incr);
-      active[1] = active[1] && ((double)nlp[1] > A.eps_pos || (double)nlr[1] > A.eps_rot) && (incr1 > A.min_incr);
+      active[0] = active[0] && (!TABLE || it + 1 < cs0.max_iter) && ((double)nlp[0] > cs0.eps_pos || (double)nlr[0] > cs0.eps_rot) && (incr0 > cs0.min_incr);
+      active[1] = active[1] && (!TABLE || it + 1 < cs1.max_iter) && ((double)nlp[1] > cs1.eps_pos || (double)nlr[1] > cs1.eps_rot) && (incr1 > cs1.min_incr);
       __syncwarp();
     }
     stamp(it, 5);
@@ -573,12 +584,13 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
       p0[i] = __shfl_sync(0xffffffffu, p[i], 0);
       gp[i] = A.gpos[clip * 3 + i] + p0[i];
     }
-    if (A.adj_joint >= 0) {
-      const float* tp = A.tgt_pos + ((size_t)clip * A.ee_stride + A.adj_slot) * 3;
+    const DpClipSetting& cs = TABLE ? S.set[n0 + c] : A.uniform;
+    if (cs.adj_joint >= 0) {
+      const float* tp = A.tgt_pos + ((size_t)clip * A.ee_stride + cs.adj_slot) * 3;
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
-        const float pj = __shfl_sync(0xffffffffu, p[i], A.adj_joint);
-        adj[i] = ((tp[i] - (A.targets_world ? A.gpos[clip * 3 + i] : 0.0f)) - pj) * A.adj_w;
+        const float pj = __shfl_sync(0xffffffffu, p[i], cs.adj_joint);
+        adj[i] = ((tp[i] - (A.targets_world ? A.gpos[clip * 3 + i] : 0.0f)) - pj) * cs.adj_w;
         gp[i] += adj[i];
       }
     }
@@ -620,12 +632,12 @@ __global__ void __launch_bounds__(kWarps * 32, 1) dp_frame_tc16_kernel(const __g
 }  // namespace
 
 cudaError_t dp_frame_tc16_launch(const DpFrameArgs& args, int num_sms, cudaStream_t stream) {
-  static std::atomic<unsigned long long> configured{0}, configured_clk{0};
+  static std::atomic<unsigned long long> configured[4];
   const size_t smem = sizeof(SmemT) + 1024;
-  const bool clk = args.phase_cycles != nullptr;
-  if (cudaError_t e = clk ? dp_ensure_smem(dp_frame_tc16_kernel<true>, smem, configured_clk) : dp_ensure_smem(dp_frame_tc16_kernel<false>, smem, configured);
-      e != cudaSuccess)
-    return e;
+  const bool clk = args.phase_cycles != nullptr, table = args.settings != nullptr;
+  auto kernel = clk ? (table ? dp_frame_tc16_kernel<true, true> : dp_frame_tc16_kernel<true, false>)
+                    : (table ? dp_frame_tc16_kernel<false, true> : dp_frame_tc16_kernel<false, false>);
+  if (cudaError_t e = dp_ensure_smem(kernel, smem, configured[2 * clk + table]); e != cudaSuccess) return e;
   // spread the clips over every SM: 4096 clips -> 28 per CTA (14 pairs dealt 4 + 4 + 3 + 3 to the groups) on 147 SMs
   DpFrameArgs a = args;
   int cpc = (args.n_clips + num_sms - 1) / num_sms;
@@ -633,7 +645,6 @@ cudaError_t dp_frame_tc16_launch(const DpFrameArgs& args, int num_sms, cudaStrea
   if (args.n_clips > num_sms * NC) cpc = NC;  // several waves anyway: use full tiles
   a.clips_per_cta = cpc;
   const int grid = (args.n_clips + cpc - 1) / cpc;
-  if (clk) dp_frame_tc16_kernel<true><<<grid, kWarps * 32, smem, stream>>>(a);
-  else dp_frame_tc16_kernel<false><<<grid, kWarps * 32, smem, stream>>>(a);
+  kernel<<<grid, kWarps * 32, smem, stream>>>(a);
   return cudaGetLastError();
 }

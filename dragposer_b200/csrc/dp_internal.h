@@ -89,3 +89,17 @@ cudaError_t dp_gather_rings_launch(const int32_t* ids, int n, const float* laten
 // otherwise own row k < window goes to slot (k + shift) % window and own row `window` to slot `window`
 cudaError_t dp_scatter_targets_launch(const float* src, int src_rows, const int32_t* ids, int n, float* dst, int dst_rows, int r0,
                                       int window, int shift, cudaStream_t st);
+// Per-clip settings on the fp32 frame kernel (dp_subset.cu): up to DP_MAX_ROW_COPIES arrays of 32-bit words copied row by row between
+// a batch and the compact rows of a subset of its clips (ids).  Rows are `width` words at `src_stride` / `dst_stride` words apart.
+struct DpRowCopy {
+  const float* src;
+  float* dst;
+  int width, src_stride, dst_stride;
+};
+#define DP_MAX_ROW_COPIES 16
+struct DpRowCopies {
+  DpRowCopy c[DP_MAX_ROW_COPIES];
+  int n;
+};
+// scatter == 0: row i of each dst <- row ids[i] of its src; scatter == 1: row ids[i] of each dst <- row i of its src
+cudaError_t dp_copy_rows_launch(const DpRowCopies& copies, const int32_t* ids, int n, int scatter, cudaStream_t st);

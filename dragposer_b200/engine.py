@@ -86,6 +86,18 @@ class RunOptions:
             float(joint_adjustment_weight), int(decoder_path), int(bool(targets_world)), int(extension_losses), float(floor_level))
 
 
+class ClipOptions:
+    """The per-clip keywords of DragPose.run (python/src/drag_pose.py:196-215), same defaults: one clip's optimiser settings in a
+    batch whose clips run with different settings (BatchedDragPose.set_clip_options; include/dp_engine.h:dp_clip_settings)."""
+
+    def __init__(self, stop_eps_pos=1e-2, stop_eps_rot=1e-2, max_iter=100, min_loss_incr=0.00001, learning_rate=1e-3,
+                 lambda_rot=1, lambda_temporal=1, joint_adjustment_indices=None, joint_adjustment_weight=0.01):
+        self.c = _lib.ClipSettings(
+            float(stop_eps_pos), float(stop_eps_rot), float(min_loss_incr), int(max_iter), float(learning_rate), float(lambda_rot),
+            float(lambda_temporal), -1 if joint_adjustment_indices is None else int(joint_adjustment_indices[0]),
+            0 if joint_adjustment_indices is None else int(joint_adjustment_indices[1]), float(joint_adjustment_weight))
+
+
 class BatchedDragPose:
     def __init__(self, pose: PoseModel, offsets, temporal: TemporalModel, max_clips: int, device: int = 0):
         self.lib = _lib.load()
@@ -190,6 +202,23 @@ class BatchedDragPose:
     def restart_pose(self, clips, dqs, global_pos, global_rot, heights, eps=None):
         """restart_clips with the latent encoded on the device from standardised dual quats (n,176) (see set_initial_pose)."""
         self.restart_clips(clips, self.encode(dqs, eps), global_pos, global_rot, heights)
+
+    def set_clip_options(self, options, which=None):
+        """Per-clip optimiser settings: clip c runs with options[which[c]] (which: (n_clips,) ints; None = options[0] for every
+        clip), bit for bit as a batch of only the clips of that entry would run with those keywords.  While they are set, the
+        per-clip keywords of run / run_frames / run_frames_device are ignored; their temporal_future_window, decoder_path,
+        targets_world, extension_losses and floor_level still apply to the whole batch.  options=None clears them.
+        set_initial_state clears them too; restart_clips keeps every clip's entry.  On the fp32 frame kernel each entry in use runs as
+        a batch of its own, one after the other (DESIGN.md section 3.4)."""
+        if options is None:
+            _lib.check(self.lib.dp_engine_set_clip_settings(self.h, 0, None, None))
+            return
+        options = list(options)
+        table = (_lib.ClipSettings * max(1, len(options)))(*[o.c for o in options])
+        idx = None if which is None else _i32(which).reshape(-1)
+        if idx is not None and idx.shape[0] != self.n_clips:
+            raise ValueError(f"which must hold one index per clip ({self.n_clips}), got {idx.shape[0]}")
+        _lib.check(self.lib.dp_engine_set_clip_settings(self.h, len(options), C.cast(table, C.c_void_p), _ptr(idx)))
 
     def clip_index(self, window):
         """Own temporal index of every clip for the next frame run with `window` (B,) -- DragPose.current_index per clip."""

@@ -52,7 +52,10 @@ typedef enum {
 
 typedef struct dp_engine dp_engine;
 
-/* Optimiser settings of one DragPose.run call (drag_pose.py:196-215). */
+/* Optimiser settings of one DragPose.run call (drag_pose.py:196-215).
+ * While a per-clip settings table is set (dp_engine_set_clip_settings), a frame reads only the batch-wide fields of this struct:
+ * temporal_future_window, decoder_path, targets_world, extension_losses and floor_level.  Its per-clip fields (those of
+ * dp_clip_settings below) are then not read, not even validated. */
 typedef struct {
   double stop_eps_pos;        /* thresholds compared in double like the Python floats */
   double stop_eps_rot;
@@ -79,6 +82,18 @@ typedef struct {
 #define DP_EXT_FORWARD 2      /* (1 - min(1, fwd_head . fwd_hips + 0.2))^2, axes flattened to the ground  drag_pose.py:137-157 */
 #define DP_EXT_HEAD_HIPS 4    /* |head - hips|^2 on the ground plane                                      drag_pose.py:159-164 */
 #define DP_EXT_HIPS_FEET 8    /* sum over the ankles (3, 7) of max(|hips - ankle|^2 - 0.2^2, 0)           drag_pose.py:166-176 */
+
+/* The per-clip subset of dp_run_params: same meaning and ranges as the fields of the same name there.  Each clip of a batch can
+ * run with its own entry of a table of these (dp_engine_set_clip_settings).  The temporal window is not part of it: the predictor
+ * runs for the whole batch at once (one schedule, one early call, one look-ahead), so the window stays in dp_run_params. */
+typedef struct {
+  double stop_eps_pos, stop_eps_rot, min_loss_incr;
+  int32_t max_iter;
+  float learning_rate, lambda_rot, lambda_temporal;
+  int32_t joint_adjust_joint, joint_adjust_slot;
+  float joint_adjust_weight;
+} dp_clip_settings;
+#define DP_MAX_CLIP_SETTINGS 32
 
 /* Pose-VAE decoder folded to three dense layers + statistics + skeleton.
  * All pointers are HOST memory, row-major, float32 unless stated. */
@@ -244,6 +259,17 @@ int dp_engine_restart_clips(dp_engine* e, int n, const int32_t* clips, const flo
 int dp_engine_get_clip_index(dp_engine* e, int window, int32_t* index);
 /* Frames until the next frame at which a restart costs no extra predictor call (0 = the next frame), or a negative dp_status. */
 int dp_engine_frames_to_boundary(const dp_engine* e, int window);
+
+/* Per-clip optimiser settings.  Clip c runs with settings[clip_setting[c]] (clip_setting: n_clips indices < n_settings, HOST
+ * pointers; NULL = setting 0 for every clip), bitwise as a batch of only the clips of that setting run with it as dp_run_params.
+ * Both frame kernels read the table; the fp32 kernel runs one gather, launch and scatter per setting in use, so a table with G
+ * settings in use costs it about G frames' kernel time (DESIGN.md section 3.4).
+ * n_settings == 0 clears the table: frames then read every field from dp_run_params again.  Every setting is validated here
+ * (max_iter in 1..DP_MAX_ITER, joint adjustment indices); each frame then checks that every clip's joint-adjustment slot is below
+ * its ee_stride and covered by its n_ee.  A failing call returns DP_ERR_ARG and leaves the engine unchanged.
+ * dp_engine_init_clips clears the table; dp_engine_restart_clips keeps every clip's index (call this again to give a restarted
+ * clip another setting).  Not a per-frame call: it waits for the frames in flight before replacing the tables they read. */
+int dp_engine_set_clip_settings(dp_engine* e, int n_settings, const dp_clip_settings* settings, const int32_t* clip_setting);
 
 /* Number of kernels launched by this engine since creation (bench "gpu_launches"). */
 long long dp_engine_launch_count(const dp_engine* e);
